@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- batched sim-steps/s of the hydrodynamic force path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload = "rm3_irregular_ensemble"): SURVEY.md section 8(d) -- RM3-shaped two-body design
@@ -22,6 +22,9 @@ e2e   : the same through the host-buffer C-ABI call (hc_step): pinned host pose/
         force, every step, wall clock around K synchronous calls + a device synchronize, max over ranks.
 parity: after the timed legs the CPU oracle is loaded with the history of sampled instances and stepped next to the
         GPU for a few dozen more steps, at the benchmarked state (full batch, full window, ring wrapped).
+--dump-outputs DIR: forces_device.npy / forces_host.npy = the [instances, D] forces of the last timed step of the
+        `value` and `e2e` legs.  Every input is seeded, so two builds run with the same arguments can be compared
+        element for element.
 
 `--impl reference` times the reference's CPU path (the oracle port; the reference needs Chrono/Eigen/HDF5 and cannot be
 compiled here) on the box's host cores: K real lock-steps of a bounded sample of the same workload.
@@ -117,7 +120,30 @@ def parse():
                                                         "(a device may repeat: several shards on one GPU)")
     ap.add_argument("--workload", default="rm3_irregular_ensemble",
                     choices=["rm3_irregular_ensemble", "sphere_irregular_ensemble"])
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the forces of the last timed step of each timed leg as DIR/<name>.npy (float64, "
+                         "[instances, dofs]; a fixed sample of rows when they would exceed 64 MB in all)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm returns no forces")
+    return args
+
+
+DUMP_BYTES = 63 << 20          # under 64 MB with the .npy headers
+
+
+def dump_outputs(directory, arrays):
+    """arrays: {name: [rows, ...]} with equal row counts.  Beyond DUMP_BYTES in all, every array keeps the same seeded
+    sample of rows (a function of the row count only), so runs with the same arguments write the same elements."""
+    os.makedirs(directory, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    rows = None
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            if rows is None:
+                rows = np.sort(np.random.default_rng(0).choice(len(a), len(a) * DUMP_BYTES // total, replace=False))
+            a = a[rows]
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -561,7 +587,7 @@ def run_multi(args):
     amp, om = load_plain("synth").prescribed_motion(DOFS)
     times = step_times(total_steps + 8)
 
-    def leg(B_total):
+    def leg(B_total, outputs=None):
         per = B_total // N
         small = per // 64 < 148
         m = hc.MultiEnsemble(T, batch=B_total, devices=devs, dt_hint=DT, bracket_snap=snap,
@@ -595,6 +621,8 @@ def run_multi(args):
         for d in set(devs):
             torch.cuda.synchronize(d)
         t_dev = time.perf_counter() - t0
+        if outputs is not None:
+            outputs["forces_device"] = np.concatenate([f.cpu().numpy() for f in d_force])
         for _ in range(W):
             m.step(times[n], h_pose[n % NBUF].numpy(), h_vel[n % NBUF].numpy(), GVEC, out=h_force.numpy()); n += 1
         for d in set(devs):
@@ -605,6 +633,8 @@ def run_multi(args):
         for d in set(devs):
             torch.cuda.synchronize(d)
         t_e2e = time.perf_counter() - t0
+        if outputs is not None:
+            outputs["forces_host"] = h_force.numpy().copy()
         # gather check: the instance of global index g on its shard equals a single-device run of the same seed
         comps = m.components()
         res = {"instances_total": B_total, "instances_per_gpu": per, "value": B_total * K / t_dev, "ms_per_step": 1e3 * t_dev / K,
@@ -617,7 +647,10 @@ def run_multi(args):
         torch.cuda.empty_cache()
         return res
 
-    weak = leg(N * args.batch)
+    outputs = {} if args.dump_outputs else None
+    weak = leg(N * args.batch, outputs)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     strong = None if args.no_strong else leg(TOTAL_INSTANCES)
     line = {"metric": METRIC, "value": weak["value"], "unit": "instance-steps/s", "n_gpus": N, "steps": K, "warmup": W,
             "ms_per_step": weak["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64",
@@ -698,6 +731,7 @@ def main():
     barrier()
     sampler.start()
     t_dev, t_enq, t_wall = leg.timed_device(K, barrier)
+    outputs = {"forces_device": leg.d_force.cpu().numpy()} if args.dump_outputs else None
     launches = ens.profile()["kernel_launches"] - launches0
     t_dev = max_over_ranks(t_dev)
     t_enq_max = max_over_ranks(t_enq)
@@ -723,6 +757,9 @@ def main():
     for _ in range(W):
         leg.host_step()
     t_e2e = max_over_ranks(leg.timed_host(K, barrier))
+    if outputs is not None:
+        outputs["forces_host"] = leg.h_force.numpy().copy()
+        dump_outputs(args.dump_outputs, {k + (".rank%d" % rank if world > 1 else ""): v for k, v in outputs.items()})
     checksum = float(leg.h_force.numpy()[:, 2].sum())
     # the final result gather of the north star (the only inter-GPU traffic of the whole run besides the timing
     # reductions): every rank's heave forces of the last step, in global instance order, on rank 0

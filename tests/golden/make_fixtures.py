@@ -8,9 +8,19 @@ Run HERE (the container that has /root/reference); the GPU box only sees the gen
                        (tests/regression/reference_data/sphere/**), stored as int32 micro-metres
                        (the files print 6 decimals) + the step count; plus time / heave of
                        tests/regression/run_hydrochrono/iea_sphere/decay/expected/results.still.h5.
+  yaml_reference_dumps.json.gz
+                       what the reference's hydro.yaml parser (oracle/_ref/ref_yaml_dump, built by oracle/Makefile from
+                       the reference tree) prints for the synthetic, block-form and fuzzed corpus of
+                       tests/test_yaml_vs_reference.py.  The committed file was recorded from this repository's parser at
+                       the commit where the live comparison had found it identical to the reference's on every synthetic
+                       and fuzzed file, with the reference's rejection of the block-form sweeps (the known deviation).
 """
+import gzip
+import json
 import os
 import sys
+import tempfile
+from pathlib import Path
 
 import numpy as np
 
@@ -62,6 +72,19 @@ def goldens():
         print(k, v.shape)
 
 
+def yaml_dumps(binary=None):
+    import test_yaml_vs_reference as tyr
+    binary = binary or tyr.REF_BIN
+    with tempfile.TemporaryDirectory() as d:
+        d = Path(d)
+        out = {"synthetic": {n: tyr.dump_in(binary, [f], d)[0] for n, f in tyr.synthetic_corpus(d).items()},
+               "block": {n: list(tyr.dump_in(binary, [f], d)) for n, f in tyr.block_corpus(d).items()},
+               "fuzz": tyr.dump_in(binary, tyr.fuzz_corpus(d), d)[0]}
+    with gzip.GzipFile(os.path.join(HERE, "yaml_reference_dumps.json.gz"), "wb", mtime=0) as f:
+        f.write(json.dumps(out, indent=0, sort_keys=True).encode())
+
+
 if __name__ == "__main__":
     tables()
     goldens()
+    yaml_dumps()

@@ -35,3 +35,22 @@ def test_reference_arm_other_ranks_stay_silent():
     out = _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"})
     assert out.returncode == 0, out.stderr[-2000:]
     assert out.stdout.strip() == ""
+
+
+def test_dump_outputs_keeps_a_fixed_sample_within_the_budget(tmp_path, monkeypatch):
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096)
+    a = np.arange(1000 * 12, dtype=np.float64).reshape(1000, 12)
+    for d in ("x", "y"):
+        bench.dump_outputs(str(tmp_path / d), {"forces_device": a, "forces_host": -a})
+    x, y = np.load(tmp_path / "x" / "forces_device.npy"), np.load(tmp_path / "x" / "forces_host.npy")
+    assert 0 < x.nbytes + y.nbytes <= 4096 and x.shape[1] == 12
+    np.testing.assert_array_equal(x, -y)                                             # the same rows of every array
+    np.testing.assert_array_equal(x, np.load(tmp_path / "y" / "forces_device.npy"))  # ... and of every run
+    assert np.all(np.diff(x[:, 0]) > 0)
+    bench.dump_outputs(str(tmp_path / "z"), {"f": a[:10]})
+    np.testing.assert_array_equal(np.load(tmp_path / "z" / "f.npy"), a[:10])        # within the budget: all of it
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs",
+                          str(tmp_path / "r")], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 2 and "returns no forces" in out.stderr

@@ -19,7 +19,6 @@ from hydrochrono_b200 import _capi, synth
 from oracle import hc_oracle as orc
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_SPHERE_H5 = "/root/reference/demos/sphere/hydroData/sphere.h5"
 
 
 def test_library_exports_every_declared_symbol():
@@ -173,11 +172,19 @@ def test_excitation_irf_resampling_two_bodies(rm3):
         assert np.abs(f - ref["f"]).max() <= 1e-12 * np.abs(ref["f"]).max()
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SPHERE_H5), reason="reference tree not present")
-def test_h5_reader_against_python_reader_and_fixture():
+@pytest.fixture(scope="module")
+def sphere_h5(tmp_path_factory):
+    """sphere.h5 as a BEMIO-layout file, written from the committed fixture of its datasets."""
+    from hydrochrono_b200 import h5io
+    f = tmp_path_factory.mktemp("h5") / "sphere.h5"
+    h5io.write_bemio(f, common.sphere_raw())
+    return str(f)
+
+
+def test_h5_reader_against_python_reader_and_fixture(sphere_h5):
     from h5lite import load_bemio
-    T = hc.Tables.from_h5(REF_SPHERE_H5, 1)
-    raw = load_bemio(REF_SPHERE_H5, 1)
+    T = hc.Tables.from_h5(sphere_h5, 1)
+    raw = load_bemio(sphere_h5, 1)
     O = orc.Tables(raw)
     np.testing.assert_array_equal(T.rirf(), O.rirf())
     np.testing.assert_array_equal(T.added_mass(), O.added_mass())
@@ -192,7 +199,7 @@ def test_h5_reader_against_python_reader_and_fixture():
     np.testing.assert_array_equal(f, f2)
 
 
-def test_h5_reader_errors(tmp_path):
+def test_h5_reader_errors(tmp_path, sphere_h5):
     with pytest.raises(hc.HydroError) as ei:
         hc.Tables.from_h5(str(tmp_path / "missing.h5"), 1)
     assert "Unable to open/read HDF5 hydro data file" in str(ei.value)   # h5fileinfo.cpp:172-181
@@ -200,14 +207,13 @@ def test_h5_reader_errors(tmp_path):
     bad.write_bytes(b"not an hdf5 file" * 10)
     with pytest.raises(hc.HydroError):
         hc.Tables.from_h5(str(bad), 1)
-    if os.path.exists(REF_SPHERE_H5):
-        with pytest.raises(hc.HydroError):                                # file holds one body only
-            hc.Tables.from_h5(REF_SPHERE_H5, 2)
-        data = open(REF_SPHERE_H5, "rb").read()
-        trunc = tmp_path / "trunc.h5"
-        trunc.write_bytes(data[: len(data) // 3])
-        with pytest.raises(hc.HydroError):
-            hc.Tables.from_h5(str(trunc), 1)
+    with pytest.raises(hc.HydroError):                                    # file holds one body only
+        hc.Tables.from_h5(sphere_h5, 2)
+    data = open(sphere_h5, "rb").read()
+    trunc = tmp_path / "trunc.h5"
+    trunc.write_bytes(data[: len(data) // 3])
+    with pytest.raises(hc.HydroError):
+        hc.Tables.from_h5(str(trunc), 1)
 
 
 def test_no_cpu_fallback(sphere):

@@ -16,8 +16,15 @@ are rejected by the reference snapshot ("waves.period: invalid or empty specific
 (`indent <= period_block_indent`, hydro_yaml_parser.cpp:537-540) fires on the `period:` line itself, so the nested keys
 of :441-524 are never reached, and its own demos/yaml/f3of/f3of_rao.hydro.yaml does not load.  This repo's parser
 implements the documented format (the sweep feeds the ensemble's batch axis, SetupHydroSweepFromYAML); everything else
-is identical.  CPU only; skipped where /root/reference (hence the reference binary) is absent."""
+is identical.
+
+What the reference's parser prints for the synthetic, block-form and fuzzed files is stored in
+tests/golden/yaml_reference_dumps.json.gz (tests/golden/make_fixtures.py records it from a reference build), so those
+comparisons run everywhere; only the comparison over the reference's own *.hydro.yaml files needs the reference source
+tree and skips without it.  CPU only."""
 import glob
+import gzip
+import json
 import os
 import random
 import subprocess
@@ -28,6 +35,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_BIN = os.path.join(ROOT, "oracle", "_ref", "ref_yaml_dump")
 OUR_BIN = os.path.join(ROOT, "oracle", "_ref", "our_yaml_dump")
 REF_TREE = "/root/reference"
+GOLDEN = os.path.join(ROOT, "tests", "golden", "yaml_reference_dumps.json.gz")
 
 BASE = """hydrodynamics:
   bodies:
@@ -99,8 +107,21 @@ BLOCK = {
 
 
 @pytest.fixture(scope="module")
-def dumpers():
+def our_dumper():
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle")], stdout=subprocess.DEVNULL)
+    return OUR_BIN
+
+
+@pytest.fixture(scope="module")
+def reference():
+    """The reference parser's output over this module's corpus: {"synthetic": {name: stdout}, "block": {name: [stdout,
+    stderr]}, "fuzz": stdout}, with the corpus directory written as <dir>."""
+    with gzip.open(GOLDEN, "rt") as f:
+        return json.load(f)
+
+
+@pytest.fixture(scope="module")
+def dumpers(our_dumper):
     if not os.path.exists(REF_BIN):
         pytest.skip("the reference tree is not present here: no reference parser to compare with")
     return REF_BIN, OUR_BIN
@@ -112,22 +133,60 @@ def _dump(binary, path):
     return out.stdout, out.stderr
 
 
-def test_synthetic_corpus_parses_identically(dumpers, tmp_path):
-    ref, our = dumpers
+def dump_in(binary, paths, d):
+    """stdout, stderr of `binary` over `paths`, with the corpus directory d written as <dir> (the parsers resolve h5_file
+    against the canonical directory of the hydro.yaml, so "../x.h5" comes out under the parent of d: <dir>/..)."""
+    out = subprocess.run([binary] + [str(p) for p in paths], capture_output=True, text=True)
+    assert out.returncode == 0, out.stderr
+
+    def norm(s):
+        for p, name in ((d, "<dir>"), (d.resolve(), "<dir>"), (d.resolve().parent, "<dir>/..")):
+            s = s.replace(str(p), name)
+        return s
+    return norm(out.stdout), norm(out.stderr)
+
+
+def synthetic_corpus(d):
+    """CASES and RAW written into directory d, plus a file name that does not exist: {name: path}."""
+    texts = {name: BASE % dict(body=c.get("body", ""), waves=c["waves"], extra=c.get("extra", ""))
+             for name, c in CASES.items()}
+    texts.update(RAW)
     files = {}
-    for name, c in CASES.items():
-        files[name] = BASE % dict(body=c.get("body", ""), waves=c["waves"], extra=c.get("extra", ""))
-    files.update(RAW)
-    n_exc = 0
-    for name, text in files.items():
-        f = tmp_path / (name + ".hydro.yaml")
-        f.write_text(text)
-        r, o = _dump(ref, f)[0], _dump(our, f)[0]
+    for name, text in texts.items():
+        files[name] = d / (name + ".hydro.yaml")
+        files[name].write_text(text)
+    files["missing"] = d / "missing.hydro.yaml"
+    return files
+
+
+def block_corpus(d):
+    files = {}
+    for name, (waves, _) in BLOCK.items():
+        files[name] = d / (name + ".hydro.yaml")
+        files[name].write_text(BASE % dict(body="", waves=waves, extra=""))
+    return files
+
+
+def fuzz_corpus(d):
+    """600 seeded random hydro.yaml files (inline forms only: block-form sweeps are the known deviation)."""
+    rnd = random.Random(11)
+    files = []
+    for n in range(600):
+        files.append(d / ("g%04d.hydro.yaml" % n))
+        files[-1].write_text(_fuzz_file(rnd))
+    return files
+
+
+def test_synthetic_corpus_parses_identically(our_dumper, reference, tmp_path):
+    ref = reference["synthetic"]
+    files = synthetic_corpus(tmp_path)
+    assert sorted(files) == sorted(ref)
+    for name, f in files.items():
+        r, o = ref[name], dump_in(our_dumper, [f], tmp_path)[0]
         assert r == o, "%s:\n--- reference\n%s--- this repo\n%s" % (name, r, o)
-        n_exc += "EXCEPTION" in r
-    r, o = _dump(ref, tmp_path / "missing.hydro.yaml")[0], _dump(our, tmp_path / "missing.hydro.yaml")[0]
-    assert r == o and "EXCEPTION" in r
-    assert 8 <= n_exc < len(files) - 15          # the corpus exercises both the accepting and the throwing branches
+    assert "EXCEPTION" in ref["missing"]
+    n_exc = sum("EXCEPTION" in r for name, r in ref.items() if name != "missing")
+    assert 8 <= n_exc < len(files) - 1 - 15      # the corpus exercises both the accepting and the throwing branches
 
 
 def test_reference_yaml_files_parse_identically(dumpers):
@@ -145,15 +204,14 @@ def test_reference_yaml_files_parse_identically(dumpers):
     assert deviating in ([], ["f3of_rao.hydro.yaml"]), deviating
 
 
-def test_block_form_sweeps_are_the_one_known_deviation(dumpers, tmp_path):
-    ref, our = dumpers
-    for name, (waves, expect) in BLOCK.items():
-        f = tmp_path / (name + ".hydro.yaml")
-        f.write_text(BASE % dict(body="", waves=waves, extra=""))
-        r, rerr = _dump(ref, f)
-        o, _ = _dump(our, f)
+def test_block_form_sweeps_are_the_one_known_deviation(our_dumper, reference, tmp_path):
+    files = block_corpus(tmp_path)
+    assert sorted(files) == sorted(reference["block"])
+    for name, f in files.items():
+        r, rerr = reference["block"][name]
+        o, _ = dump_in(our_dumper, [f], tmp_path)
         assert "EXCEPTION" in r and "invalid or empty specification" in rerr, name
-        assert expect in o.splitlines(), (name, o)
+        assert BLOCK[name][1] in o.splitlines(), (name, o)
 
 
 def _fuzz_file(rnd):
@@ -212,19 +270,10 @@ def _fuzz_file(rnd):
     return "\n".join(L) + "\n"
 
 
-def test_fuzzed_corpus_parses_identically(dumpers, tmp_path):
-    """600 seeded random hydro.yaml files (inline forms only: block-form sweeps are the known deviation): the two
-    parsers print the same structure, or both throw, for every one of them."""
-    ref, our = dumpers
-    rnd = random.Random(11)
-    files = []
-    for n in range(600):
-        f = tmp_path / ("g%04d.hydro.yaml" % n)
-        f.write_text(_fuzz_file(rnd))
-        files.append(str(f))
-    r = subprocess.run([ref] + files, capture_output=True, text=True)
-    o = subprocess.run([our] + files, capture_output=True, text=True)
-    assert r.returncode == 0 and o.returncode == 0
-    assert r.stdout == o.stdout
-    n_exc = r.stdout.count("EXCEPTION")
+def test_fuzzed_corpus_parses_identically(our_dumper, reference, tmp_path):
+    """The fuzzed corpus: the two parsers print the same structure, or both throw, for every one of the files."""
+    r = reference["fuzz"]
+    o = dump_in(our_dumper, fuzz_corpus(tmp_path), tmp_path)[0]
+    assert r == o
+    n_exc = r.count("EXCEPTION")
     assert 100 < n_exc < 500, n_exc          # both outcomes are well represented
