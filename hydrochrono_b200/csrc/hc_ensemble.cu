@@ -428,7 +428,13 @@ void hc_ensemble::setup_radiation_chunks() {
         chunk = pick_chunk(L, tiles * (templated ? 1 : D / 6), sm_count, occ, size_t(110) * 1024, smem_of, D, 4);
     }
     chunk = std::max(1, std::min(chunk, L));
-    while (chunk > 1 && (D == 6 || D == 12) && radiation_smem_bytes(D, chunk) > 200 * 1024) chunk /= 2;
+    // clamp with the shared memory of the kernel that launch_radiation will pick (a user rad_chunk is not checked
+    // elsewhere): the DMMA kernel stages 16-row fragments, more per lag than the FMA and hybrid kernels
+    auto launch_smem = [&](int c) -> size_t {
+        if (rad_mma) return radiation_mma_smem_bytes(c);
+        return (D == 6 || D == 12) ? radiation_smem_bytes(D, c) : 0;
+    };
+    while (chunk > 1 && launch_smem(chunk) > 200 * 1024) chunk /= 2;
     rad_chunk = chunk;
     rad_nchunk = (L + chunk - 1) / chunk;
     d_rad_partial.alloc(size_t(rad_nchunk) * D * Bp);
@@ -1400,7 +1406,11 @@ void hc_ensemble::setup_excitation_groups(double simulation_dt) {
         if (chunk <= 0)
             chunk = pick_chunk(max_Le, tiles * ngroups, e->sm_count, 2, size_t(110) * 1024, excitation_smem_bytes,
                                e->exc_ndmax, 16);
-        e->exc_chunk = std::min(chunk, std::max(1, max_Le));
+        chunk = std::min(chunk, std::max(1, max_Le));
+        // a user exc_chunk must still fit k_excitation's dynamic shared memory (200 KB attribute), as the radiation
+        // chunk does
+        while (chunk > 1 && excitation_smem_bytes(e->exc_ndmax, chunk) > 200 * 1024) chunk /= 2;
+        e->exc_chunk = chunk;
     }
     int chunk0 = 0;
     for (int g = 0; g < ngroups; ++g) {
