@@ -105,6 +105,18 @@ def _dp(a):
     return a.ctypes.data_as(_capi.dp) if a is not None else None
 
 
+def _kin_points(points, batch):
+    pts = _f64(points)
+    if pts.ndim != 3 or pts.shape[0] != batch or pts.shape[2] != 3:
+        raise ValueError("points must be [batch][P][3]")
+    return pts
+
+
+def _kin_outputs(pts):
+    B, P = pts.shape[:2]
+    return np.empty((B, P)), np.empty((B, P, 3)), np.empty((B, P, 3))
+
+
 def _ptr(x):
     """Address of a numpy array / torch tensor / raw integer pointer."""
     if x is None:
@@ -408,6 +420,23 @@ class Ensemble:
         _check(lib.hc_waves_force_at_time(self._h, float(t), _dp(out)))
         return out
 
+    def wave_kinematics(self, t, points, mwl=0.0, wheeler=False):
+        """Water elevation, particle velocity and acceleration of every instance's wave at its own points
+        (WaveBase::GetElevation / GetVelocity / GetAcceleration, on the device): points [B][P][3] ->
+        (eta [B][P], vel [B][P][3], acc [B][P][3]).  Irregular eta is not ramped; see hc_waves_kinematics_at_time."""
+        pts = _kin_points(points, self.batch)
+        eta, vel, acc = _kin_outputs(pts)
+        _check(lib.hc_waves_kinematics_at_time(self._h, float(t), pts.shape[1], _dp(pts), float(mwl), int(bool(wheeler)),
+                                               _dp(eta), _dp(vel), _dp(acc)))
+        return eta, vel, acc
+
+    def wave_kinematics_device(self, t, n_points, d_points, d_eta=None, d_vel=None, d_acc=None, mwl=0.0, wheeler=False):
+        """wave_kinematics on device buffers (torch CUDA tensors or raw addresses; any output may be None):
+        d_points [B][n_points][3], d_eta [B][n_points], d_vel / d_acc [B][n_points][3]; asynchronous on the
+        ensemble stream."""
+        _check(lib.hc_waves_kinematics_at_time_device(self._h, float(t), int(n_points), _ptr(d_points), float(mwl),
+                                                      int(bool(wheeler)), _ptr(d_eta), _ptr(d_vel), _ptr(d_acc)))
+
     def refresh_rirf(self):
         _check(lib.hc_ensemble_refresh_rirf(self._h))
 
@@ -557,6 +586,14 @@ class MultiEnsemble:
         n = len(d_pose)
         arr = [(C.c_void_p * n)(*[_ptr(x).value for x in lst]) for lst in (d_pose, d_vel, d_force)]
         _check(lib.hc_multi_step_device(self._h, float(t), arr[0], arr[1], _dp(g), arr[2]))
+
+    def wave_kinematics(self, t, points, mwl=0.0, wheeler=False):
+        """Ensemble.wave_kinematics over every shard: points [B][P][3] in global instance order."""
+        pts = _kin_points(points, self.batch)
+        eta, vel, acc = _kin_outputs(pts)
+        _check(lib.hc_multi_waves_kinematics_at_time(self._h, float(t), pts.shape[1], _dp(pts), float(mwl),
+                                                     int(bool(wheeler)), _dp(eta), _dp(vel), _dp(acc)))
+        return eta, vel, acc
 
     def components(self):
         shape = (self.batch, self.dofs)

@@ -110,6 +110,8 @@ SIGNATURES = {
     "hc_step_device": (C.c_int, [vp, C.c_double, vp, vp, dp, vp, ip]),
     "hc_get_components": (C.c_int, [vp, dp, dp, dp]),
     "hc_waves_force_at_time": (C.c_int, [vp, C.c_double, dp]),
+    "hc_waves_kinematics_at_time": (C.c_int, [vp, C.c_double, C.c_int, dp, C.c_double, C.c_int, dp, dp, dp]),
+    "hc_waves_kinematics_at_time_device": (C.c_int, [vp, C.c_double, C.c_int, vp, C.c_double, C.c_int, vp, vp, vp]),
     "hc_ensemble_refresh_rirf": (C.c_int, [vp]),
     "hc_sync": (C.c_int, [vp]),
     "hc_ensemble_join": (C.c_int, [vp]),
@@ -141,6 +143,7 @@ SIGNATURES = {
     "hc_multi_waves_irregular_series": (C.c_int, [vp, C.c_double, C.c_int, dp, dp, C.c_int]),
     "hc_multi_step": (C.c_int, [vp, C.c_double, vp, vp, dp, vp, ip]),
     "hc_multi_step_device": (C.c_int, [vp, C.c_double, C.POINTER(vp), C.POINTER(vp), dp, C.POINTER(vp)]),
+    "hc_multi_waves_kinematics_at_time": (C.c_int, [vp, C.c_double, C.c_int, dp, C.c_double, C.c_int, dp, dp, dp]),
     "hc_multi_get_components": (C.c_int, [vp, dp, dp, dp]),
     "hc_multi_sync": (C.c_int, [vp]),
     "hc_multi_reset": (C.c_int, [vp]),

@@ -185,6 +185,7 @@ struct hc_ensemble {
     int wave_mode = 0;
     DevBuf<double> d_reg_amp, d_reg_omega, d_reg_mag, d_reg_phase;
     std::vector<double> reg_mag_h, reg_phase_h, reg_k_h;   // [count][D], [count][D], [count]
+    std::vector<double> reg_amp_h, reg_omega_h, reg_wave_phase_h;   // [count] each (the wave itself: kinematics)
     int reg_count = 0;
     // irregular
     hc_irregular_params ip{};
@@ -210,6 +211,18 @@ struct hc_ensemble {
     std::vector<double> phases_h;     // [B][nf]
     bool per_instance_spectrum = false;
     int n_eta = 0, nf = 0;
+    void pack_irregular(std::vector<double>& amp, std::vector<double>& ph) const;
+    // water kinematics (hc_waves_kinematics_at_time): the wave's components staged on the first call (per-instance
+    // phases and amplitudes [nf][Bp], 8 B x nf x Bp each), released whenever the waves are set again
+    DevBuf<double> d_kin_comp, d_kin_amp, d_kin_phase, d_kin_io;
+    bool kin_staged = false;
+    void stage_kinematics();
+    void release_kinematics() {
+        d_kin_comp.release(); d_kin_amp.release(); d_kin_phase.release(); d_kin_io.release();
+        kin_staged = false;
+    }
+    void enqueue_kinematics(double t, int n_points, const double* d_points, double mwl, int wheeler, double* d_eta,
+                            double* d_vel, double* d_acc);
     // excitation look-ahead (state-independent wave force evaluated kLaT predicted steps at a time)
     bool la_enabled = false;
     double la_dt = 0.0;
@@ -1324,6 +1337,7 @@ hc_status hc_waves_none(hc_ensemble* e) {
     e->use_device();
     CUDA_CHECK(cudaStreamSynchronize(e->stream));
     e->wave_mode = 0;
+    e->release_kinematics();
     e->drop_graph();
     return HC_OK;
     HC_GUARD_END
@@ -1369,7 +1383,11 @@ hc_status hc_waves_regular(hc_ensemble* e, int count, const double* amplitude, c
         for (int d = 0; d < D; ++d) mag[size_t(d) * Bp + b] = e->reg_mag_h[size_t(i) * D + d];
         for (int r = 0; r < 6; ++r) ph[size_t(r) * Bp + b] = e->reg_phase_h[size_t(i) * D + r];   // body 0 (quirk, :323)
     }
-    (void)phase;  // regular_wave_phase_ is not used by the force (only by eta / kinematics)
+    // regular_wave_phase_ is not used by the force, only by eta / kinematics
+    e->reg_amp_h.assign(amplitude, amplitude + count);
+    e->reg_omega_h.assign(omega, omega + count);
+    if (phase) e->reg_wave_phase_h.assign(phase, phase + count); else e->reg_wave_phase_h.assign(count, 0.0);
+    e->release_kinematics();
     e->d_reg_amp.upload(amp); e->d_reg_omega.upload(om); e->d_reg_mag.upload(mag); e->d_reg_phase.upload(ph);
     e->wave_mode = 1;
     e->drop_graph();
@@ -1388,6 +1406,7 @@ void hc_irregular_default_params(hc_irregular_params* p) {
 void hc_ensemble::setup_excitation_groups(double simulation_dt) {
     hc_ensemble* e = this;
     const hc_tables& T = *e->T;
+    release_kinematics();
     irf = resample_excitation_irf(T, simulation_dt);
     // group bodies that share one IRF time grid bit-for-bit (the usual case: one BEMIO run)
     groups.clear();
@@ -1443,6 +1462,21 @@ void hc_ensemble::setup_excitation_groups(double simulation_dt) {
     e->drop_graph();
 }
 
+// Device layout of the irregular components (k_eta, k_wave_kinematics): phases [nf][Bp], amplitudes sqrt(2 S df)
+// [nf][Bp] when the spectrum is per instance, else [nf]; padded lanes zero.
+void hc_ensemble::pack_irregular(std::vector<double>& amp, std::vector<double>& ph) const {
+    amp.assign(per_instance_spectrum ? size_t(nf) * Bp : size_t(nf), 0.0);
+    ph.assign(size_t(nf) * Bp, 0.0);
+    const int nS = per_instance_spectrum ? B : 1;
+    for (int s = 0; s < nS; ++s)
+        for (int i = 0; i < nf; ++i) {
+            const double a = std::sqrt(2 * S_h[size_t(s) * nf + i] * widths_h[i]);     // GetEtaIrregular (:39)
+            if (per_instance_spectrum) amp[size_t(i) * Bp + s] = a; else amp[i] = a;
+        }
+    for (int b = 0; b < B; ++b)
+        for (int i = 0; i < nf; ++i) ph[size_t(i) * Bp + b] = phases_h[size_t(b) * nf + i];
+}
+
 hc_status hc_waves_irregular(hc_ensemble* e, const hc_irregular_params* p, const int* seeds, const double* Hs_arr,
                              const double* Tp_arr) {
     HC_GUARD_BEGIN
@@ -1492,25 +1526,22 @@ hc_status hc_waves_irregular(hc_ensemble* e, const hc_irregular_params* p, const
     e->per_instance_spectrum = (Hs_arr != nullptr) || (Tp_arr != nullptr);
     const int nS = e->per_instance_spectrum ? B : 1;
     e->S_h.resize(size_t(nS) * nf);
-    std::vector<double> amp(e->per_instance_spectrum ? size_t(nf) * Bp : size_t(nf), 0.0);
     for (int s = 0; s < nS; ++s) {
         const double Hs = Hs_arr ? Hs_arr[s] : p->wave_height;
         const double Tp = Tp_arr ? Tp_arr[s] : p->wave_period;
         dvec S = jonswap(e->freqs_h, Hs, Tp, p->peak_enhancement_factor, p->is_normalized != 0);
         std::copy(S.begin(), S.end(), e->S_h.begin() + size_t(s) * nf);
-        for (int i = 0; i < nf; ++i) {
-            const double a = std::sqrt(2 * S[i] * e->widths_h[i]);      // GetEtaIrregular (:39)
-            if (e->per_instance_spectrum) amp[size_t(i) * Bp + s] = a; else amp[i] = a;
-        }
     }
     e->phases_h.resize(size_t(B) * nf);
-    std::vector<double> ph(size_t(nf) * Bp, 0.0);
     for (int b = 0; b < B; ++b) {
         dvec v = random_phases(seeds ? seeds[b] : p->seed, nf);
         std::copy(v.begin(), v.end(), e->phases_h.begin() + size_t(b) * nf);
-        for (int i = 0; i < nf; ++i) ph[size_t(i) * Bp + b] = v[i];
     }
-    e->d_omega.upload(omega); e->d_amp.upload(amp); e->d_phase.upload(ph);
+    {
+        std::vector<double> amp, ph;
+        e->pack_irregular(amp, ph);
+        e->d_omega.upload(omega); e->d_amp.upload(amp); e->d_phase.upload(ph);
+    }
 
     // --- eta synthesis on the device (wave_types.cpp:27-59,750-769) ---
     EtaArgs ea{};
@@ -1822,6 +1853,99 @@ hc_status hc_waves_force_at_time(hc_ensemble* e, double t, double* out) {
     e->prof.kernel_launches += 2 + (e->wave_mode == 2 ? (long long)e->groups.size() : 0);
     return HC_OK;
     HC_GUARD_END
+}
+
+// WaveBase::GetElevation / GetVelocity / GetAcceleration for every instance at its own points; like
+// hc_waves_force_at_time it reads no eta window or history and touches no force cache.
+hc_status hc_waves_kinematics_at_time_device(hc_ensemble* e, double t, int n_points, const double* d_points, double mwl,
+                                             int wheeler_stretching, double* d_eta, double* d_velocity,
+                                             double* d_acceleration) {
+    HC_GUARD_BEGIN
+    if (n_points < 1 || !d_points) fail(HC_ERR_INVALID, "n_points must be positive and points non-null");
+    e->use_device();
+    e->enqueue_kinematics(t, n_points, d_points, mwl, wheeler_stretching, d_eta, d_velocity, d_acceleration);
+    return HC_OK;
+    HC_GUARD_END
+}
+
+hc_status hc_waves_kinematics_at_time(hc_ensemble* e, double t, int n_points, const double* points, double mwl,
+                                      int wheeler_stretching, double* eta, double* velocity, double* acceleration) {
+    HC_GUARD_BEGIN
+    if (n_points < 1 || !points) fail(HC_ERR_INVALID, "n_points must be positive and points non-null");
+    e->use_device();
+    const size_t n = size_t(e->B) * n_points;
+    // one device block: points [n][3] | eta [n] | velocity [n][3] | acceleration [n][3]
+    if (e->d_kin_io.n < 10 * n) e->d_kin_io.alloc(10 * n, false);
+    double* dp = e->d_kin_io.p;
+    double* de = dp + 3 * n;
+    double* dv = de + n;
+    double* da = dv + 3 * n;
+    CUDA_CHECK(cudaMemcpyAsync(dp, points, 3 * n * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+    e->enqueue_kinematics(t, n_points, dp, mwl, wheeler_stretching, eta ? de : nullptr, velocity ? dv : nullptr,
+                          acceleration ? da : nullptr);
+    if (eta) CUDA_CHECK(cudaMemcpyAsync(eta, de, n * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    if (velocity) CUDA_CHECK(cudaMemcpyAsync(velocity, dv, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    if (acceleration)
+        CUDA_CHECK(cudaMemcpyAsync(acceleration, da, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    CUDA_CHECK(cudaStreamSynchronize(e->stream));
+    return HC_OK;
+    HC_GUARD_END
+}
+
+// Components of the current waves for k_wave_kinematics.  omega, k, the branch flag and sinh(k depth) are computed here
+// with the reference's expressions (wave_types.cpp:66-83): the same doubles the host arithmetic uses.
+void hc_ensemble::stage_kinematics() {
+    const double depth = T->depth;
+    auto deep = [depth](double k) { return (2 * M_PI / k > depth || k * depth > 500.0) ? 1.0 : 0.0; };
+    auto put = [](std::vector<double>& c, size_t stride, size_t j, double om, double k, double dp, double shkd, double A,
+                  double ph) {
+        c[kKinOmega * stride + j] = om; c[kKinK * stride + j] = k; c[kKinDeep * stride + j] = dp;
+        c[kKinSinhKd * stride + j] = shkd; c[kKinAmp * stride + j] = A; c[kKinPhase * stride + j] = ph;
+    };
+    if (wave_mode == 1) {
+        std::vector<double> c(size_t(kKinFields) * Bp, 0.0);
+        for (int b = 0; b < B; ++b) {
+            const int i = reg_count == 1 ? 0 : b;
+            const double k = reg_k_h[i];
+            put(c, Bp, b, reg_omega_h[i], k, deep(k), std::sinh(k * depth), reg_amp_h[i], reg_wave_phase_h[i]);
+        }
+        d_kin_comp.upload(c);
+    } else {
+        std::vector<double> amp, ph;
+        pack_irregular(amp, ph);
+        std::vector<double> c(size_t(kKinFields) * nf, 0.0);
+        for (int i = 0; i < nf; ++i) {
+            const double k = wavenumbers_h[i];
+            put(c, nf, i, 2 * M_PI * freqs_h[i], k, deep(k), std::sinh(k * depth), per_instance_spectrum ? 0.0 : amp[i],
+                0.0);
+        }
+        d_kin_comp.upload(c);
+        d_kin_phase.upload(ph);
+        if (per_instance_spectrum) d_kin_amp.upload(amp);
+    }
+    kin_staged = true;
+}
+
+void hc_ensemble::enqueue_kinematics(double t, int n_points, const double* d_points, double mwl, int wheeler,
+                                     double* d_eta, double* d_vel, double* d_acc) {
+    const size_t n = size_t(B) * n_points;
+    if (wave_mode == 0 || (wave_mode == 2 && nf == 0)) {
+        // NoWave, an imported eta series, or no sea state: the reference sums over empty component vectors
+        if (d_eta) CUDA_CHECK(cudaMemsetAsync(d_eta, 0, n * sizeof(double), stream));
+        if (d_vel) CUDA_CHECK(cudaMemsetAsync(d_vel, 0, 3 * n * sizeof(double), stream));
+        if (d_acc) CUDA_CHECK(cudaMemsetAsync(d_acc, 0, 3 * n * sizeof(double), stream));
+        return;
+    }
+    if (!kin_staged) stage_kinematics();
+    KinArgs a{};
+    a.points = d_points; a.eta = d_eta; a.vel = d_vel; a.acc = d_acc;
+    a.comp = d_kin_comp.p; a.amp = d_kin_amp.p; a.phase = d_kin_phase.p;
+    a.t = t; a.depth = T->depth; a.mwl = mwl;
+    a.B = B; a.Bp = Bp; a.P = n_points; a.nf = nf;
+    a.regular = wave_mode == 1;
+    a.wheeler = (wave_mode == 2 && wheeler) ? 1 : 0;
+    CUDA_CHECK(launch_wave_kinematics(a, sm_count, stream));
+    prof.kernel_launches += 1;
 }
 
 // Re-stages the radiation kernel after hc_tables_set_convolution_mode was called on the ensemble's tables.

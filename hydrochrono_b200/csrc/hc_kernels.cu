@@ -21,6 +21,8 @@
 //                 (no k_prestep level); a warp, not a thread, per (dof, instance) in the finalize
 //   k_eta         free-surface elevation synthesis for every realisation
 //                                                        src/wave_types.cpp:14-59,717-769
+//   k_wave_kinematics  elevation, particle velocity and acceleration at given points for every instance (off the step
+//                 path)                                  src/wave_types.cpp:14-160,301-313,515-550
 //   k_added_mass_mv  R += c * M * w, batched             src/chloadaddedmass.cpp:55-71
 //
 // Layout: lanes <-> instances.  History ring hist[slot][dof][instance] and eta[sample][instance] are
@@ -1691,6 +1693,131 @@ __global__ void __launch_bounds__(128) k_eta(const EtaArgs a) {
 }
 
 // ------------------------------------------------------------------------------------------
+// k_wave_kinematics: WaveBase::GetElevation / GetVelocity / GetAcceleration (wave_types.cpp:14-160,301-313,515-550)
+// for every instance at its own points.  One thread = one instance x PPT points of it (blockIdx.y strides over point
+// groups), so every phase it loads serves all of them.  Per-component fields are staged in shared memory, per-instance
+// phases / amplitudes are [nf][Bp] as in k_eta (one coalesced load per warp and component).  The reference's
+// expressions with their left-to-right products, every operation rounded on its own (no contraction):
+//   arg = (k x - omega t) + phi,  eta += A cos(arg) in ascending i  (at x = 0: bit for bit k_eta's sum)
+//   deep water:  v = (omega A) e^{kz} (cos, sin),  a = ((omega omega) A) e^{kz} sin, ((-omega omega) A) e^{kz} cos
+//   finite:      e^{kz} -> cosh(k (z + depth)) / sinh(k depth) in x,  sinh(k (z + depth)) / sinh(k depth) in z
+// sincos returns bit for bit the cos of k_eta (same reduction and polynomial), so the single pass shares its eta.
+// ------------------------------------------------------------------------------------------
+struct KinAcc { double eta, vx, vz, ax, az; };
+
+__device__ __forceinline__ double kin_arg(double om, double k, double ph, double t, double x) {
+    return __dadd_rn(__dsub_rn(__dmul_rn(k, x), __dmul_rn(om, t)), ph);
+}
+
+// one component's share at one point; z = position.z - mwl (stretched for Wheeler)
+__device__ __forceinline__ void kin_add(KinAcc& r, double om, double k, bool deep, double shkd, double A, double ph,
+                                        double t, double depth, double x, double z, bool with_eta) {
+    double s, c;
+    sincos(kin_arg(om, k, ph, t, x), &s, &c);
+    if (with_eta) r.eta = __dadd_rn(r.eta, __dmul_rn(A, c));
+    const double oa = __dmul_rn(om, A);
+    const double ooa = __dmul_rn(__dmul_rn(om, om), A);
+    const double nooa = __dmul_rn(__dmul_rn(-om, om), A);
+    double vx, vz, ax, az;
+    if (deep) {                                                         // wave_types.cpp:71-76, :103-108
+        const double e = exp(__dmul_rn(k, z));
+        vx = __dmul_rn(oa, e); vz = vx;
+        ax = __dmul_rn(ooa, e); az = __dmul_rn(nooa, e);
+    } else {                                                            // :77-83, :109-115
+        const double kz = __dmul_rn(k, __dadd_rn(z, depth));
+        const double ch = cosh(kz), sh = sinh(kz);
+        vx = __ddiv_rn(__dmul_rn(oa, ch), shkd); vz = __ddiv_rn(__dmul_rn(oa, sh), shkd);
+        ax = __ddiv_rn(__dmul_rn(ooa, ch), shkd); az = __ddiv_rn(__dmul_rn(nooa, sh), shkd);
+    }
+    r.vx = __dadd_rn(r.vx, __dmul_rn(vx, c));
+    r.vz = __dadd_rn(r.vz, __dmul_rn(vz, s));
+    r.ax = __dadd_rn(r.ax, __dmul_rn(ax, s));
+    r.az = __dadd_rn(r.az, __dmul_rn(az, c));
+}
+
+// one pass over the irregular components: ETA_ONLY = GetEtaIrregular (Wheeler's first pass), else the kinematics
+template <int PPT, bool ETA_ONLY>
+__device__ __forceinline__ void kin_irregular_pass(const KinArgs& a, double (*s_c)[kKinChunk], int b, int np,
+                                                   const double* x, const double* z, KinAcc* r, bool with_eta) {
+    for (int i0 = 0; i0 < a.nf; i0 += kKinChunk) {
+        const int n = min(kKinChunk, a.nf - i0);
+        __syncthreads();
+        for (int q = threadIdx.x; q < n; q += blockDim.x)
+#pragma unroll
+            for (int f = 0; f < kKinPhase; ++f) s_c[f][q] = a.comp[(size_t)f * a.nf + i0 + q];
+        __syncthreads();
+        if (np == 0) continue;
+        for (int q = 0; q < n; ++q) {
+            const size_t ib = (size_t)(i0 + q) * a.Bp + b;
+            const double A = a.amp ? a.amp[ib] : s_c[kKinAmp][q];
+            const double ph = a.phase[ib];
+            const double om = s_c[kKinOmega][q], k = s_c[kKinK][q];
+#pragma unroll
+            for (int j = 0; j < PPT; ++j) {
+                if (j >= np) break;
+                if (ETA_ONLY) r[j].eta = __dadd_rn(r[j].eta, __dmul_rn(A, cos(kin_arg(om, k, ph, a.t, x[j]))));
+                else kin_add(r[j], om, k, s_c[kKinDeep][q] != 0.0, s_c[kKinSinhKd][q], A, ph, a.t, a.depth, x[j], z[j],
+                             with_eta);
+            }
+        }
+    }
+}
+
+template <int PPT, bool REGULAR>
+__global__ void __launch_bounds__(128) k_wave_kinematics(const KinArgs a) {
+    __shared__ double s_c[kKinPhase][kKinChunk];
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    const int groups = (a.P + PPT - 1) / PPT;
+    for (int g = blockIdx.y; g < groups; g += gridDim.y) {             // uniform per CTA (syncthreads inside)
+        const int p0 = g * PPT;
+        const int np = b < a.B ? min(PPT, a.P - p0) : 0;
+        double x[PPT], z[PPT];
+        KinAcc r[PPT];
+#pragma unroll
+        for (int j = 0; j < PPT; ++j) {
+            x[j] = 0.0; z[j] = 0.0;
+            r[j] = KinAcc{0.0, 0.0, 0.0, 0.0, 0.0};
+            if (j < np) {
+                const double* p = a.points + ((size_t)b * a.P + p0 + j) * 3;
+                x[j] = p[0];
+                z[j] = __dsub_rn(p[2], a.mwl);                          // z_pos = position.z - mwl
+            }
+        }
+        if (REGULAR) {                                                  // RegularWave: one component, never stretched
+            if (np > 0) {
+                const double* c = a.comp + b;
+                const size_t s = a.Bp;
+                const double om = c[kKinOmega * s], k = c[kKinK * s], shkd = c[kKinSinhKd * s];
+                const double A = c[kKinAmp * s], ph = c[kKinPhase * s];
+                const bool deep = c[kKinDeep * s] != 0.0;
+#pragma unroll
+                for (int j = 0; j < PPT; ++j)
+                    if (j < np) kin_add(r[j], om, k, deep, shkd, A, ph, a.t, a.depth, x[j], z[j], true);
+            }
+        } else {
+            if (a.wheeler) {                                            // wave_types.cpp:530-533
+                kin_irregular_pass<PPT, true>(a, s_c, b, np, x, z, r, true);
+#pragma unroll
+                for (int j = 0; j < PPT; ++j) {
+                    const double e = r[j].eta;
+                    // position_stretched.z = depth (z_pos - eta) / (depth + eta); GetWaterVelocity subtracts mwl again
+                    z[j] = __dsub_rn(__ddiv_rn(__dmul_rn(a.depth, __dsub_rn(z[j], e)), __dadd_rn(a.depth, e)), a.mwl);
+                }
+            }
+            kin_irregular_pass<PPT, false>(a, s_c, b, np, x, z, r, !a.wheeler);
+        }
+#pragma unroll
+        for (int j = 0; j < PPT; ++j) {
+            if (j >= np) break;
+            const size_t o = (size_t)b * a.P + p0 + j;
+            if (a.eta) a.eta[o] = r[j].eta;
+            if (a.vel) { a.vel[3 * o] = r[j].vx; a.vel[3 * o + 1] = 0.0; a.vel[3 * o + 2] = r[j].vz; }
+            if (a.acc) { a.acc[3 * o] = r[j].ax; a.acc[3 * o + 1] = 0.0; a.acc[3 * o + 2] = r[j].az; }
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // k_added_mass_mv: R[b][i] += sum_j (c*M[i][j]) * w[b][j];  M is the padded n_sys x n_sys matrix.
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128) k_added_mass_mv(const double* __restrict__ M, int n_sys, int D, double c,
@@ -1892,6 +2019,21 @@ cudaError_t launch_finalize(const FinalizeArgs& a, const HydrostaticTables& hs, 
 cudaError_t launch_eta(const EtaArgs& a, cudaStream_t st) {
     dim3 grid((a.Bp + 127) / 128, (a.n_eta + kEtaKT - 1) / kEtaKT);
     k_eta<<<grid, 128, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+// Points per thread: as many as keep at least two CTAs per SM (more phase reuse per thread while the grid still fills
+// the GPU), one when even that leaves SMs short.
+cudaError_t launch_wave_kinematics(const KinArgs& a, int sm_count, cudaStream_t st) {
+    const int xb = (a.B + 127) / 128;
+    auto groups = [&](int ppt) { return (a.P + ppt - 1) / ppt; };
+    const int ppt = (long long)xb * groups(kKinPts) >= 2LL * sm_count ? kKinPts
+                  : (long long)xb * groups(2) >= 2LL * sm_count ? 2 : 1;
+    const dim3 grid(xb, std::min(groups(ppt), 65535));
+    if (a.regular) k_wave_kinematics<1, true><<<dim3(xb, std::min(groups(1), 65535)), 128, 0, st>>>(a);
+    else if (ppt == kKinPts) k_wave_kinematics<kKinPts, false><<<grid, 128, 0, st>>>(a);
+    else if (ppt == 2) k_wave_kinematics<2, false><<<grid, 128, 0, st>>>(a);
+    else k_wave_kinematics<1, false><<<grid, 128, 0, st>>>(a);
     return cudaGetLastError();
 }
 

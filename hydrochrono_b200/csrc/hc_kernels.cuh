@@ -112,6 +112,29 @@ struct EtaArgs {
     int n_eta, nf, Bp, amp_per_instance;
 };
 
+// Water kinematics at caller-given points for every instance (k_wave_kinematics).  Lanes map to instances; each thread
+// evaluates up to kKinPts points of its instance, further points go to blockIdx.y.
+constexpr int kKinPts = 4;
+constexpr int kKinChunk = 128;        // components staged in shared memory at a time
+// rows of KinArgs::comp: omega, wavenumber, deep-water flag (1.0 / 0.0), sinh(k depth), amplitude, phase
+enum { kKinOmega = 0, kKinK, kKinDeep, kKinSinhKd, kKinAmp, kKinPhase, kKinFields };
+struct KinArgs {
+    const double* points;     // [B][P][3]
+    double* eta;              // [B][P]    or null
+    double* vel;              // [B][P][3] or null
+    double* acc;              // [B][P][3] or null
+    // irregular waves: comp = [kKinFields][nf] per component (amplitude row = the shared spectrum's, phase row unused),
+    // phase = [nf][Bp] per instance, amp = [nf][Bp] per instance or null when the spectrum is shared.
+    // regular waves: comp = [kKinFields][Bp], one component per instance; amp and phase unused.
+    const double* comp;
+    const double* amp;
+    const double* phase;
+    double t, depth, mwl;
+    int B, Bp, P, nf;
+    int regular;
+    int wheeler;              // irregular only: z' = depth (z - mwl - eta) / (depth + eta)
+};
+
 struct PrestepArgs {
     const StepHeader* hdr;
     double* hist;          // [cap][D][Bp]
@@ -160,6 +183,7 @@ cudaError_t launch_excitation(const ExcitationArgs& a, const ExcGroup& g, const 
 cudaError_t launch_finalize(const FinalizeArgs& a, const HydrostaticTables& hs, const FinalizeGroups& eg,
                             cudaStream_t st);
 cudaError_t launch_eta(const EtaArgs& a, cudaStream_t st);
+cudaError_t launch_wave_kinematics(const KinArgs& a, int sm_count, cudaStream_t st);
 // ---- excitation look-ahead: the wave force of T consecutive (predicted) step times in one pass over eta ----
 // Which finalize kernel serves an ensemble (depends only on its size and chunking, never on the step):
 constexpr int kFinalizeWarpMaxB = 8;          // up to this many instances: k_finalize_warp (a warp per (dof, instance))

@@ -219,6 +219,17 @@ hc_status hc_multi_step_device(hc_multi_ensemble* m, double t, const double* con
     });
 }
 
+hc_status hc_multi_waves_kinematics_at_time(hc_multi_ensemble* m, double t, int n_points, const double* points, double mwl,
+                                            int wheeler_stretching, double* eta, double* velocity, double* acceleration) {
+    if (n_points < 1 || !points) { hc::set_last_error("n_points must be positive and points non-null"); return HC_ERR_INVALID; }
+    return m->run([=](hc::Worker& k) {
+        const size_t off = size_t(k.first) * n_points;
+        return hc_waves_kinematics_at_time(k.ens, t, n_points, points + 3 * off, mwl, wheeler_stretching,
+                                           eta ? eta + off : nullptr, velocity ? velocity + 3 * off : nullptr,
+                                           acceleration ? acceleration + 3 * off : nullptr);
+    });
+}
+
 hc_status hc_multi_get_components(hc_multi_ensemble* m, double* hs, double* rad, double* waves) {
     const int D = m->D;
     return m->run([=](hc::Worker& k) {

@@ -41,6 +41,14 @@ class TestHydroEnsemble {
     void AddWavesIrregular(const IrregularWaveParams& base, const std::vector<int>& seeds, const std::vector<double>& Hs,
                            const std::vector<double>& Tp);
 
+    // water elevation, particle velocity and acceleration of every instance's wave at its own points on the device
+    // (WaveBase::GetElevation / GetVelocity / GetAcceleration, hc_waves_kinematics_at_time): points [B][n_points][3]
+    // in, eta [B][n_points], vel / acc [B][n_points][3] out (resized; any may be null).  Wheeler stretching as the
+    // IrregularWaveParams::wave_stretching_ given to AddWavesIrregular.  Irregular eta is not ramped.  Not a force
+    // evaluation: the force cache and DeviceEvaluations() are untouched.
+    void GetWaveKinematics(double t, int n_points, const std::vector<double>& points, std::vector<double>* eta,
+                           std::vector<double>* vel, std::vector<double>* acc, double mwl = 0.0);
+
     // total force on body b (1-based) of instance inst in DoF i; one batched device evaluation per time value
     double CoordinateFuncForInstance(int inst, int b, int i);
     // the three components of the last evaluation, [B][6N] each
@@ -60,6 +68,7 @@ class TestHydroEnsemble {
     hc_ensemble* ens_ = nullptr;
     std::vector<double> pose_, vel_, force_;
     double prev_time_ = -1.0;
+    bool wave_stretching_ = false;
     long long evaluations_ = 0;
     std::vector<std::shared_ptr<chrono::ChLoadContainer>> load_containers_;
     std::vector<std::shared_ptr<ChLoadAddedMass>> added_mass_;

@@ -89,13 +89,17 @@ TestHydroEnsemble::~TestHydroEnsemble() {
     if (ens_) hc_ensemble_destroy(ens_);
 }
 
-void TestHydroEnsemble::AddWavesNone() { hc_throw_on_error(hc_waves_none(ens_)); }
+void TestHydroEnsemble::AddWavesNone() {
+    hc_throw_on_error(hc_waves_none(ens_));
+    wave_stretching_ = false;
+}
 
 void TestHydroEnsemble::AddWavesRegular(const std::vector<double>& amplitude, const std::vector<double>& omega) {
     const size_t B = size_t(Batch());
     if (amplitude.size() != omega.size() || !(amplitude.size() == 1 || amplitude.size() == B))
         throw std::runtime_error("TestHydroEnsemble::AddWavesRegular: need 1 or B (amplitude, omega) pairs");
     hc_throw_on_error(hc_waves_regular(ens_, int(amplitude.size()), amplitude.data(), omega.data(), nullptr));
+    wave_stretching_ = false;
 }
 
 void TestHydroEnsemble::AddWavesIrregular(const IrregularWaveParams& p, const std::vector<int>& seeds,
@@ -112,6 +116,20 @@ void TestHydroEnsemble::AddWavesIrregular(const IrregularWaveParams& p, const st
     q.is_normalized = p.is_normalized_ ? 1 : 0; q.seed = p.seed_;
     hc_throw_on_error(hc_waves_irregular(ens_, &q, seeds.empty() ? nullptr : seeds.data(), Hs.empty() ? nullptr : Hs.data(),
                                          Tp.empty() ? nullptr : Tp.data()));
+    wave_stretching_ = p.wave_stretching_;
+}
+
+void TestHydroEnsemble::GetWaveKinematics(double t, int n_points, const std::vector<double>& points, std::vector<double>* eta,
+                                          std::vector<double>* vel, std::vector<double>* acc, double mwl) {
+    const size_t n = size_t(Batch()) * size_t(n_points > 0 ? n_points : 0);
+    if (n_points < 1 || points.size() != 3 * n)
+        throw std::runtime_error("TestHydroEnsemble::GetWaveKinematics: points must be [B][n_points][3], n_points >= 1");
+    if (eta) eta->resize(n);
+    if (vel) vel->resize(3 * n);
+    if (acc) acc->resize(3 * n);
+    hc_throw_on_error(hc_waves_kinematics_at_time(ens_, t, n_points, points.data(), mwl, wave_stretching_ ? 1 : 0,
+                                                  eta ? eta->data() : nullptr, vel ? vel->data() : nullptr,
+                                                  acc ? acc->data() : nullptr));
 }
 
 // One batched device step at the current Chrono time with the state every system holds at this moment.

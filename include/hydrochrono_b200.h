@@ -259,6 +259,29 @@ HC_API hc_status hc_get_components(hc_ensemble* e, double* hydrostatic, double* 
 /* WaveBase::GetForceAtTime(t) (src/wave_types.cpp:257-264,315-327,552-570) for every instance, host [B][6N]:
  * the wave excitation force alone at an arbitrary time; does not touch the velocity history or the force cache. */
 HC_API hc_status hc_waves_force_at_time(hc_ensemble* e, double t, double* waves);
+/* Water kinematics of every instance's own wave at its own points: WaveBase::GetElevation / GetVelocity /
+ * GetAcceleration (src/wave_types.cpp:14-160,301-313,515-550) evaluated on the device (k_wave_kinematics).
+ * points [B][P][3] (x, y, z) in, eta [B][P], velocity and acceleration [B][P][3] out; any output may be NULL.
+ * - NoWave (hc_waves_none, a fresh ensemble), an imported eta series (hc_waves_irregular_series) or irregular waves
+ *   without a sea state: every output is zero (the reference sums over empty component vectors).
+ * - Regular waves: the instance's amplitude, omega, phase and wavenumber; Wheeler stretching is never applied.
+ * - Irregular waves: the nf spectral components, amplitudes sqrt(2 S df) and phases of the instance.  eta is NOT
+ *   ramped (GetEtaIrregular has no ramp), so during the ramp it differs from the synthesised series that
+ *   hc_waves_irregular_eta returns; at x = 0 after the ramp it equals that series' samples bit for bit.  With
+ *   wheeler_stretching != 0, velocity and acceleration are taken at z' = depth (z - mwl - eta) / (depth + eta).
+ * - Deep-water branch per component when 2 pi / k > depth or k depth > 500, finite depth otherwise.
+ * Any t is allowed: the call reads no eta window and no history, touches no force cache and is not a force
+ * evaluation.  The first call after the waves were set stages the components on the device (irregular waves:
+ * per-instance phases, and per-instance amplitudes when the sea state is per instance, 8 nf B bytes each); they are
+ * released when the waves are set again or the ensemble is destroyed.
+ * n_points < 1 or points == NULL: HC_ERR_INVALID.  Synchronous at return. */
+HC_API hc_status hc_waves_kinematics_at_time(hc_ensemble* e, double t, int n_points, const double* points,
+                                             double mwl, int wheeler_stretching,
+                                             double* eta, double* velocity, double* acceleration);
+/* The same with device pointers on the ensemble's device, asynchronous on the ensemble's stream. */
+HC_API hc_status hc_waves_kinematics_at_time_device(hc_ensemble* e, double t, int n_points, const double* d_points,
+                                                    double mwl, int wheeler_stretching,
+                                                    double* d_eta, double* d_velocity, double* d_acceleration);
 /* Re-stage the radiation kernel after hc_tables_set_convolution_mode() changed the ensemble's tables. */
 HC_API hc_status hc_ensemble_refresh_rirf(hc_ensemble* e);
 HC_API hc_status hc_sync(hc_ensemble* e);
@@ -368,6 +391,11 @@ HC_API hc_status hc_multi_step(hc_multi_ensemble* m, double t, const double* pos
  * shards' streams (hc_multi_sync waits). */
 HC_API hc_status hc_multi_step_device(hc_multi_ensemble* m, double t, const double* const* d_pose, const double* const* d_vel,
                                       const double g_vec[3], double* const* d_force);
+/* hc_waves_kinematics_at_time for every shard at once: host arrays in global instance order (points [B][P][3], eta
+ * [B][P], velocity / acceleration [B][P][3]); each shard fills its slice concurrently.  Synchronous at return. */
+HC_API hc_status hc_multi_waves_kinematics_at_time(hc_multi_ensemble* m, double t, int n_points, const double* points,
+                                                   double mwl, int wheeler_stretching,
+                                                   double* eta, double* velocity, double* acceleration);
 /* Final gather of the three force components of the last evaluation, host [B][6N] each (may be NULL). */
 HC_API hc_status hc_multi_get_components(hc_multi_ensemble* m, double* hydrostatic, double* radiation, double* waves);
 HC_API hc_status hc_multi_sync(hc_multi_ensemble* m);
