@@ -128,6 +128,55 @@ def _ptr(x):
     return C.c_void_p(x.ctypes.data)
 
 
+_SCHEMES = {"euler": 0, "hht": 1, 0: 0, 1: 1}
+
+
+def _sim_params(dofs, batch, n_steps, dt, t0, scheme, record_every, gvec, mass, inertia, free_dof, pto_damping,
+                pto_stiffness):
+    """hc_sim_params and the arrays it points to (kept alive by the caller through the returned tuple)."""
+    if scheme not in _SCHEMES:
+        raise ValueError("scheme must be 'euler' or 'hht'")
+    N = dofs // 6
+    keep = {"mass": _f64(np.broadcast_to(np.asarray(mass, dtype=np.float64), (N,))),
+            "inertia": _f64(np.broadcast_to(np.asarray(inertia, dtype=np.float64), (N, 3)))}
+    if free_dof is not None:
+        keep["free"] = np.ascontiguousarray(np.broadcast_to(np.asarray(free_dof).astype(np.int32), (dofs,)))
+    for name, x in (("c", pto_damping), ("k", pto_stiffness)):
+        if x is not None:
+            keep[name] = _f64(np.broadcast_to(np.asarray(x, dtype=np.float64), (batch, dofs)))
+    p = _capi.SimParams()
+    p.scheme, p.t0, p.dt, p.n_steps, p.record_every = _SCHEMES[scheme], float(t0), float(dt), int(n_steps), int(record_every)
+    for i, v in enumerate(gvec):
+        p.g[i] = float(v)
+    p.mass, p.inertia = _dp(keep["mass"]), _dp(keep["inertia"])
+    p.free_dof = keep["free"].ctypes.data_as(_capi.ip) if "free" in keep else None
+    p.pto_damping, p.pto_stiffness = _dp(keep.get("c")), _dp(keep.get("k"))
+    return p, keep
+
+
+def _simulate_host(fn, handle, batch, dofs, pose0, vel0, n_steps, record_every, record, energy, p):
+    pose = _f64(pose0).reshape(batch, dofs).copy()
+    vel = np.zeros((batch, dofs)) if vel0 is None else _f64(vel0).reshape(batch, dofs).copy()
+    n_rec = n_steps // max(int(record_every), 1) if record else 0
+    times, rp, rv = np.empty(n_rec), np.empty((n_rec, batch, dofs)), np.empty((n_rec, batch, dofs))
+    e = np.empty((batch, dofs)) if energy else None
+    done = C.c_int()
+    st = fn(handle, C.byref(p), _dp(pose), _dp(vel), _dp(times) if n_rec else None, _dp(rp) if n_rec else None,
+            _dp(rv) if n_rec else None, _dp(e), C.byref(done))
+    return st, SimResult(times, rp, rv, e, done.value, pose, vel)
+
+
+class SimResult(tuple):
+    """(times, pose, vel, pto_energy, steps_done) of a device-stepped run: times [n_rec] and pose / vel
+    [n_rec][B][6N] are the recorded states (state after step (k+1) record_every), pto_energy [B][6N] (or None);
+    final_pose / final_vel [B][6N] are the state after the last completed step."""
+
+    def __new__(cls, times, pose, vel, energy, steps_done, final_pose, final_vel):
+        r = super().__new__(cls, (times, pose, vel, energy, steps_done))
+        r.final_pose, r.final_vel = final_pose, final_vel
+        return r
+
+
 class Tables:
     """HydroData (reference include/hydroc/h5fileinfo.h:35-226)."""
 
@@ -437,6 +486,36 @@ class Ensemble:
         _check(lib.hc_waves_kinematics_at_time_device(self._h, float(t), int(n_points), _ptr(d_points), float(mwl),
                                                       int(bool(wheeler)), _ptr(d_eta), _ptr(d_vel), _ptr(d_acc)))
 
+    def simulate(self, pose0, n_steps, dt, mass, inertia, vel0=None, t0=0.0, scheme="euler", record_every=1,
+                 gvec=(0.0, 0.0, -9.81), free_dof=None, pto_damping=None, pto_stiffness=None, record=True,
+                 energy=True, check=True):
+        """Advances every instance n_steps on the device (hc_ensemble_simulate): rigid bodies with each DoF free or
+        locked to ground (free_dof [6N], None = all free), gravity, optional linear PTO per instance and DoF
+        (pto_damping / pto_stiffness [B][6N] or broadcastable).  scheme 'euler' (linearised Euler) or 'hht'
+        (HHT-alpha, alpha = -0.2).  Returns SimResult (times, pose, vel, pto_energy, steps_done) as numpy arrays;
+        with check=False a force-path error is returned as result.status instead of raised."""
+        p, keep = _sim_params(self.dofs, self.batch, n_steps, dt, t0, scheme, record_every, gvec, mass, inertia,
+                              free_dof, pto_damping, pto_stiffness)
+        st, res = _simulate_host(lib.hc_ensemble_simulate, self._h, self.batch, self.dofs, pose0, vel0, n_steps,
+                                 record_every, record, energy, p)
+        res.status = st
+        if check:
+            _check(st)
+        return res
+
+    def simulate_device(self, d_pose, d_vel, n_steps, dt, mass, inertia, t0=0.0, scheme="euler", record_every=1,
+                        gvec=(0.0, 0.0, -9.81), free_dof=None, pto_damping=None, pto_stiffness=None, d_rec_t=None,
+                        d_rec_pose=None, d_rec_vel=None, d_pto_energy=None):
+        """simulate on device buffers (torch CUDA tensors or raw addresses): d_pose / d_vel [B][6N] in: initial
+        state, out: final state; d_rec_t [n_rec], d_rec_pose / d_rec_vel [n_rec][B][6N], d_pto_energy [B][6N], any
+        may be None.  Asynchronous on the ensemble stream.  Returns steps_done (force-path errors are raised)."""
+        p, keep = _sim_params(self.dofs, self.batch, n_steps, dt, t0, scheme, record_every, gvec, mass, inertia,
+                              free_dof, pto_damping, pto_stiffness)
+        done = C.c_int()
+        _check(lib.hc_ensemble_simulate_device(self._h, C.byref(p), _ptr(d_pose), _ptr(d_vel), _ptr(d_rec_t),
+                                               _ptr(d_rec_pose), _ptr(d_rec_vel), _ptr(d_pto_energy), C.byref(done)))
+        return done.value
+
     def refresh_rirf(self):
         _check(lib.hc_ensemble_refresh_rirf(self._h))
 
@@ -594,6 +673,20 @@ class MultiEnsemble:
         _check(lib.hc_multi_waves_kinematics_at_time(self._h, float(t), pts.shape[1], _dp(pts), float(mwl),
                                                      int(bool(wheeler)), _dp(eta), _dp(vel), _dp(acc)))
         return eta, vel, acc
+
+    def simulate(self, pose0, n_steps, dt, mass, inertia, vel0=None, t0=0.0, scheme="euler", record_every=1,
+                 gvec=(0.0, 0.0, -9.81), free_dof=None, pto_damping=None, pto_stiffness=None, record=True,
+                 energy=True, check=True):
+        """Ensemble.simulate over every shard (hc_multi_ensemble_simulate), arrays in global instance order; each
+        shard runs its whole loop on its own worker thread."""
+        p, keep = _sim_params(self.dofs, self.batch, n_steps, dt, t0, scheme, record_every, gvec, mass, inertia,
+                              free_dof, pto_damping, pto_stiffness)
+        st, res = _simulate_host(lib.hc_multi_ensemble_simulate, self._h, self.batch, self.dofs, pose0, vel0, n_steps,
+                                 record_every, record, energy, p)
+        res.status = st
+        if check:
+            _check(st)
+        return res
 
     def components(self):
         shape = (self.batch, self.dofs)

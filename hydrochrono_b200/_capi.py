@@ -57,6 +57,12 @@ class ProfileStats(C.Structure):
                 ("eta_synthesis_seconds", C.c_double), ("step_seconds", C.c_double), ("kernel_launches", C.c_longlong)]
 
 
+class SimParams(C.Structure):
+    _fields_ = [("scheme", C.c_int), ("t0", C.c_double), ("dt", C.c_double), ("n_steps", C.c_int),
+                ("record_every", C.c_int), ("g", C.c_double * 3), ("mass", dp), ("inertia", dp), ("free_dof", ip),
+                ("pto_damping", dp), ("pto_stiffness", dp)]
+
+
 # every symbol include/hydrochrono_b200.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "hc_last_error": (C.c_char_p, []),
@@ -112,6 +118,8 @@ SIGNATURES = {
     "hc_waves_force_at_time": (C.c_int, [vp, C.c_double, dp]),
     "hc_waves_kinematics_at_time": (C.c_int, [vp, C.c_double, C.c_int, dp, C.c_double, C.c_int, dp, dp, dp]),
     "hc_waves_kinematics_at_time_device": (C.c_int, [vp, C.c_double, C.c_int, vp, C.c_double, C.c_int, vp, vp, vp]),
+    "hc_ensemble_simulate": (C.c_int, [vp, C.POINTER(SimParams), dp, dp, dp, dp, dp, dp, ip]),
+    "hc_ensemble_simulate_device": (C.c_int, [vp, C.POINTER(SimParams), vp, vp, vp, vp, vp, vp, ip]),
     "hc_ensemble_refresh_rirf": (C.c_int, [vp]),
     "hc_sync": (C.c_int, [vp]),
     "hc_ensemble_join": (C.c_int, [vp]),
@@ -144,6 +152,7 @@ SIGNATURES = {
     "hc_multi_step": (C.c_int, [vp, C.c_double, vp, vp, dp, vp, ip]),
     "hc_multi_step_device": (C.c_int, [vp, C.c_double, C.POINTER(vp), C.POINTER(vp), dp, C.POINTER(vp)]),
     "hc_multi_waves_kinematics_at_time": (C.c_int, [vp, C.c_double, C.c_int, dp, C.c_double, C.c_int, dp, dp, dp]),
+    "hc_multi_ensemble_simulate": (C.c_int, [vp, C.POINTER(SimParams), dp, dp, dp, dp, dp, dp, ip]),
     "hc_multi_get_components": (C.c_int, [vp, dp, dp, dp]),
     "hc_multi_sync": (C.c_int, [vp]),
     "hc_multi_reset": (C.c_int, [vp]),

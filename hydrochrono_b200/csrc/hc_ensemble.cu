@@ -181,6 +181,18 @@ struct hc_ensemble {
 
     PinBuf h_pose, h_vel, h_force;
 
+    // device-side stepping (hc_ensemble_simulate).  d_sim holds [B][D] slots: evaluation pose / velocity ping-pong pairs
+    // (what the force path reads), HHT state and history, the spring rest pose and the energy of the host variant;
+    // d_simq the state and predictor orientations [B][N][4] each.  The force path's kernels read the evaluation state
+    // through the step header on the ensemble's stream only (the look-ahead passes on the side streams read the history
+    // ring), so a buffer is free again once the next step's k_body_step has read it.
+    enum { kSimPose0 = 0, kSimPose1, kSimVel0, kSimVel1, kSimX, kSimV, kSimFn, kSimAn, kSimX0, kSimEnergy, kSimSlots };
+    DevBuf<double> d_sim, d_simq, d_minv, d_pto, d_rec;
+    PinBuf h_rec;
+    size_t h_rec_bytes = 0;
+    bool sim_q_valid = false;                     // d_simq holds the orientations of the last run's final state
+    double* sim(int slot) { return d_sim.p + size_t(slot) * B * D; }
+
     // waves
     int wave_mode = 0;
     DevBuf<double> d_reg_amp, d_reg_omega, d_reg_mag, d_reg_phase;
@@ -1946,6 +1958,207 @@ void hc_ensemble::enqueue_kinematics(double t, int n_points, const double* d_poi
     a.wheeler = (wave_mode == 2 && wheeler) ? 1 : 0;
     CUDA_CHECK(launch_wave_kinematics(a, sm_count, stream));
     prof.kernel_launches += 1;
+}
+
+// ---- device-side stepping ----------------------------------------------------------------
+// Inverse of diag(m, m, m, Ixx, Iyy, Izz) + A_inf restricted to the free DoFs (Gauss-Jordan, partial pivoting), zero
+// rows and columns at locked DoFs.
+static std::vector<double> sim_inverse_mass(const hc_tables* T, const hc_sim_params& p, unsigned long long free_mask) {
+    const int D = T->D;
+    std::vector<int> idx;
+    for (int i = 0; i < D; ++i) if ((free_mask >> i) & 1ull) idx.push_back(i);
+    const int n = int(idx.size());
+    std::vector<double> A(size_t(n) * 2 * n, 0.0);
+    for (int r = 0; r < n; ++r) {
+        const int i = idx[r], b = i / 6, k = i % 6;
+        for (int c = 0; c < n; ++c) {
+            const int j = idx[c];
+            double m = (i == j) ? (k < 3 ? p.mass[b] : p.inertia[3 * b + k - 3]) : 0.0;
+            m += T->body[b].ainf[size_t(k) * D + j];
+            A[size_t(r) * 2 * n + c] = m;
+        }
+        A[size_t(r) * 2 * n + n + r] = 1.0;
+    }
+    for (int c = 0; c < n; ++c) {
+        int piv = c;
+        for (int r = c + 1; r < n; ++r)
+            if (std::fabs(A[size_t(r) * 2 * n + c]) > std::fabs(A[size_t(piv) * 2 * n + c])) piv = r;
+        const double d = A[size_t(piv) * 2 * n + c];
+        if (d == 0.0 || !std::isfinite(d)) fail(HC_ERR_INVALID, "hc_ensemble_simulate: singular free-DoF mass matrix");
+        if (piv != c) for (int k = 0; k < 2 * n; ++k) std::swap(A[size_t(c) * 2 * n + k], A[size_t(piv) * 2 * n + k]);
+        for (int k = 0; k < 2 * n; ++k) A[size_t(c) * 2 * n + k] /= d;
+        for (int r = 0; r < n; ++r) {
+            const double f = A[size_t(r) * 2 * n + c];
+            if (r == c || f == 0.0) continue;
+            for (int k = 0; k < 2 * n; ++k) A[size_t(r) * 2 * n + k] -= f * A[size_t(c) * 2 * n + k];
+        }
+    }
+    std::vector<double> Minv(size_t(D) * D, 0.0);
+    for (int r = 0; r < n; ++r)
+        for (int c = 0; c < n; ++c) {
+            const double v = A[size_t(r) * 2 * n + n + c];
+            if (!std::isfinite(v)) fail(HC_ERR_INVALID, "hc_ensemble_simulate: singular free-DoF mass matrix");
+            Minv[size_t(idx[r]) * D + idx[c]] = v;
+        }
+    return Minv;
+}
+
+// host = true: pose, vel, rec_*, energy are host memory (records through a bounded device buffer, copied out in chunks;
+// record k of rec_pose / rec_vel starts at element k * rec_stride).  host = false: device memory, rec_stride = B D.
+static hc_status sim_run(hc_ensemble* e, const hc_sim_params* p, bool host, double* pose, double* vel, double* rec_t,
+                         double* rec_pose, double* rec_vel, size_t rec_stride, double* energy, int* steps_done) {
+    HC_GUARD_BEGIN
+    if (steps_done) *steps_done = 0;
+    if (!p || !pose || !vel) fail(HC_ERR_INVALID, "hc_ensemble_simulate: null params, pose or vel");
+    if (p->n_steps < 1 || p->record_every < 1) fail(HC_ERR_INVALID, "hc_ensemble_simulate: n_steps and record_every must be >= 1");
+    if (!(p->dt > 0.0)) fail(HC_ERR_INVALID, "hc_ensemble_simulate: dt must be > 0");
+    if (!p->mass || !p->inertia) fail(HC_ERR_INVALID, "hc_ensemble_simulate: mass and inertia are required");
+    if (p->scheme != 0 && p->scheme != 1) fail(HC_ERR_INVALID, "hc_ensemble_simulate: scheme must be 0 (Euler) or 1 (HHT)");
+    e->use_device();
+    const int B = e->B, D = e->D, N = e->N;
+    const size_t bd = size_t(B) * D, bytes = bd * sizeof(double);
+    unsigned long long free_mask = 0;
+    for (int i = 0; i < D; ++i) if (!p->free_dof || p->free_dof[i]) free_mask |= 1ull << i;
+    const std::vector<double> Minv = sim_inverse_mass(e->T, *p, free_mask);
+    cudaStream_t st = e->stream;
+    if (e->d_sim.n != size_t(hc_ensemble::kSimSlots) * bd) { e->d_sim.alloc(size_t(hc_ensemble::kSimSlots) * bd); e->sim_q_valid = false; }
+    if (e->d_simq.n != size_t(8) * B * N) { e->d_simq.alloc(size_t(8) * B * N); e->sim_q_valid = false; }
+    if (e->d_minv.n != size_t(D) * D) e->d_minv.alloc(size_t(D) * D);
+    // pageable sources: the runtime stages them at the call, so the host vectors may go out of scope at once
+    CUDA_CHECK(cudaMemcpyAsync(e->d_minv.p, Minv.data(), Minv.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    const bool has_c = p->pto_damping != nullptr, has_k = p->pto_stiffness != nullptr;
+    if ((has_c || has_k) && e->d_pto.n != 2 * bd) e->d_pto.alloc(2 * bd);
+    if (has_c) CUDA_CHECK(cudaMemcpyAsync(e->d_pto.p, p->pto_damping, bytes, cudaMemcpyHostToDevice, st));
+    if (has_k) CUDA_CHECK(cudaMemcpyAsync(e->d_pto.p + bd, p->pto_stiffness, bytes, cudaMemcpyHostToDevice, st));
+    const cudaMemcpyKind in = host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+    const cudaMemcpyKind out = host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+    CUDA_CHECK(cudaMemcpyAsync(e->sim(hc_ensemble::kSimPose0), pose, bytes, in, st));
+    CUDA_CHECK(cudaMemcpyAsync(e->sim(hc_ensemble::kSimVel0), vel, bytes, in, st));
+    double* d_energy = energy ? (host ? e->sim(hc_ensemble::kSimEnergy) : energy) : nullptr;
+    if (d_energy) CUDA_CHECK(cudaMemsetAsync(d_energy, 0, bytes, st));
+
+    // records: device variant straight into the caller's arrays, host variant through a chunk of R records
+    const int n_rec = p->n_steps / p->record_every;
+    const bool want_rec = (rec_pose || rec_vel) && n_rec > 0;
+    int R = n_rec;
+    if (host && want_rec) {
+        R = int(std::max<size_t>(1, std::min<size_t>(size_t(n_rec), (size_t(64) << 20) / (2 * bytes))));
+        if (e->d_rec.n < 2 * size_t(R) * bd) e->d_rec.alloc(2 * size_t(R) * bd, false);
+        if (e->h_rec_bytes < 2 * size_t(R) * bytes) { e->h_rec.alloc(2 * size_t(R) * bytes); e->h_rec_bytes = 2 * size_t(R) * bytes; }
+    }
+    int chunk_first = 0, chunk_len = 0;
+    auto flush = [&]() {
+        if (!host || chunk_len == 0) return;
+        double* hp = static_cast<double*>(e->h_rec.p);
+        CUDA_CHECK(cudaMemcpyAsync(hp, e->d_rec.p, size_t(chunk_len) * bytes, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaMemcpyAsync(hp + size_t(R) * bd, e->d_rec.p + size_t(R) * bd, size_t(chunk_len) * bytes,
+                                   cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        for (int k = 0; k < chunk_len; ++k) {
+            if (rec_pose) std::memcpy(rec_pose + size_t(chunk_first + k) * rec_stride, hp + size_t(k) * bd, bytes);
+            if (rec_vel) std::memcpy(rec_vel + size_t(chunk_first + k) * rec_stride, hp + size_t(R + k) * bd, bytes);
+        }
+        chunk_first += chunk_len;
+        chunk_len = 0;
+    };
+
+    BodyStepArgs a{};
+    a.force = e->d_force.p;
+    a.q = e->d_simq.p; a.qe = e->d_simq.p + size_t(4) * B * N;
+    a.Minv = e->d_minv.p;
+    a.pto_c = has_c ? e->d_pto.p : nullptr;
+    a.pto_k = has_k ? e->d_pto.p + bd : nullptr;
+    a.x0 = has_k ? e->sim(hc_ensemble::kSimX0) : nullptr;
+    for (int k = 0; k < 3; ++k) a.g[k] = p->g[k];
+    for (int b = 0; b < N; ++b) a.mass[b] = p->mass[b];
+    a.dt = p->dt; a.free_mask = free_mask; a.B = B; a.N = N; a.D = D;
+    const bool hht = p->scheme == 1;
+    if (hht) {
+        a.sx = e->sim(hc_ensemble::kSimX); a.sv = e->sim(hc_ensemble::kSimV);
+        a.Fn = e->sim(hc_ensemble::kSimFn); a.an = e->sim(hc_ensemble::kSimAn);
+    }
+    auto evp = [&](int i) { return e->sim(hc_ensemble::kSimPose0 + i); };
+    auto evv = [&](int i) { return e->sim(hc_ensemble::kSimVel0 + i); };
+    auto launch = [&](int mode, int cur) {
+        a.pose_in = evp(cur); a.vel_in = evv(cur);
+        a.pose_out = evp(mode == kBodyInit ? cur : cur ^ 1); a.vel_out = evv(mode == kBodyInit ? cur : cur ^ 1);
+        CUDA_CHECK(launch_body_step(a, mode, st));
+        e->prof.kernel_launches += 1;
+    };
+    a.keep_q = e->sim_q_valid ? 1 : 0;
+    launch(kBodyInit, 0);
+    e->sim_q_valid = true;
+    a.keep_q = 0;
+
+    std::vector<double> times(static_cast<size_t>(n_rec), 0.0);
+    double t = p->t0;
+    int cur = 0, done = 0;
+    hc_status status = HC_OK;
+    if (hht) {
+        status = hc_step_device(e, t, evp(0), evv(0), p->g, e->d_force.p, nullptr);     // StepHHTBegin's F_0
+        if (status == HC_OK) { launch(kBodyHHTStart, 0); cur = 1; }
+    }
+    for (int n = 0; status == HC_OK && n < p->n_steps; ++n) {
+        if (hht) t += p->dt;
+        status = hc_step_device(e, t, evp(cur), evv(cur), p->g, e->d_force.p, nullptr);
+        if (status != HC_OK) break;
+        if (!hht) t += p->dt;
+        const bool rec_step = n_rec > 0 && (n + 1) % p->record_every == 0;
+        const int k = (n + 1) / p->record_every - 1;
+        if (rec_step) times[size_t(k)] = t;
+        const bool rec = want_rec && rec_step;
+        a.energy = d_energy;
+        a.rec_pose = a.rec_vel = nullptr;
+        if (rec) {
+            if (host) {
+                a.rec_pose = e->d_rec.p + size_t(chunk_len) * bd;
+                a.rec_vel = e->d_rec.p + size_t(R + chunk_len) * bd;
+            } else {
+                a.rec_pose = rec_pose ? rec_pose + size_t(k) * rec_stride : nullptr;
+                a.rec_vel = rec_vel ? rec_vel + size_t(k) * rec_stride : nullptr;
+            }
+        }
+        launch(hht ? kBodyHHTStep : kBodyEuler, cur);
+        cur ^= 1;
+        done = n + 1;
+        if (rec && host && ++chunk_len == R) flush();
+    }
+    const std::string msg = status == HC_OK ? std::string() : std::string(hc_last_error());
+    flush();
+    // final state: Euler = the evaluation buffer of the next step; HHT = the state slots (the evaluation buffer holds
+    // the predictor)
+    CUDA_CHECK(cudaMemcpyAsync(pose, hht ? e->sim(hc_ensemble::kSimX) : evp(cur), bytes, out, st));
+    CUDA_CHECK(cudaMemcpyAsync(vel, hht ? e->sim(hc_ensemble::kSimV) : evv(cur), bytes, out, st));
+    if (energy && host) CUDA_CHECK(cudaMemcpyAsync(energy, d_energy, bytes, cudaMemcpyDeviceToHost, st));
+    const size_t n_done_rec = size_t(done / p->record_every);
+    if (rec_t && n_done_rec > 0) {
+        if (host) std::memcpy(rec_t, times.data(), n_done_rec * sizeof(double));
+        else CUDA_CHECK(cudaMemcpyAsync(rec_t, times.data(), n_done_rec * sizeof(double), cudaMemcpyHostToDevice, st));
+    }
+    if (host) CUDA_CHECK(cudaStreamSynchronize(st));
+    if (steps_done) *steps_done = done;
+    if (status != HC_OK) fail(status, msg);
+    return HC_OK;
+    HC_GUARD_END
+}
+
+hc_status hc_ensemble_simulate(hc_ensemble* e, const hc_sim_params* p, double* pose, double* vel, double* rec_t,
+                               double* rec_pose, double* rec_vel, double* pto_energy, int* steps_done) {
+    return sim_run(e, p, true, pose, vel, rec_t, rec_pose, rec_vel, size_t(e->B) * e->D, pto_energy, steps_done);
+}
+
+hc_status hc_ensemble_simulate_device(hc_ensemble* e, const hc_sim_params* p, double* d_pose, double* d_vel,
+                                      double* d_rec_t, double* d_rec_pose, double* d_rec_vel, double* d_pto_energy,
+                                      int* steps_done) {
+    return sim_run(e, p, false, d_pose, d_vel, d_rec_t, d_rec_pose, d_rec_vel, size_t(e->B) * e->D, d_pto_energy,
+                   steps_done);
+}
+
+// hc_multi_ensemble_simulate: a shard's slice of global-order host arrays (records keep the global record stride)
+hc_status hc_ensemble_simulate_strided(hc_ensemble* e, const hc_sim_params* p, double* pose, double* vel, double* rec_t,
+                                       double* rec_pose, double* rec_vel, size_t rec_stride, double* pto_energy,
+                                       int* steps_done) {
+    return sim_run(e, p, true, pose, vel, rec_t, rec_pose, rec_vel, rec_stride, pto_energy, steps_done);
 }
 
 // Re-stages the radiation kernel after hc_tables_set_convolution_mode was called on the ensemble's tables.

@@ -97,3 +97,9 @@ hc_tables* load_bemio_h5(const char* path, int num_bodies);
 hc_tables* tables_from_desc(const hc_tables_desc& d);
 
 }  // namespace hc
+
+// hc_multi_ensemble_simulate's per-shard call (hc_ensemble.cu): hc_ensemble_simulate on host arrays whose record k
+// starts at element k * rec_stride (a shard's slice of global-order records)
+extern "C" hc_status hc_ensemble_simulate_strided(hc_ensemble* e, const hc_sim_params* p, double* pose, double* vel,
+                                                  double* rec_t, double* rec_pose, double* rec_vel, size_t rec_stride,
+                                                  double* pto_energy, int* steps_done);

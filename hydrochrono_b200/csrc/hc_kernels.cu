@@ -2183,4 +2183,177 @@ cudaError_t launch_added_mass_mv(const double* M, int n_sys, int D, double c, co
     return cudaGetLastError();
 }
 
+// ---- k_body_step: the chrono_compat stepper (host/src/chrono_compat.cpp) for free / ground-locked bodies ----
+// Every product and sum is rounded on its own (no FMA contraction), in the operand order of the C++ stand-in.
+namespace {
+__device__ __forceinline__ double mul(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ double add(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ double sub(double a, double b) { return __dsub_rn(a, b); }
+
+struct Quat { double e0, e1, e2, e3; };
+
+__device__ __forceinline__ Quat qmul(const Quat& a, const Quat& q) {      // ChQuaterniond::operator*
+    return {sub(sub(sub(mul(a.e0, q.e0), mul(a.e1, q.e1)), mul(a.e2, q.e2)), mul(a.e3, q.e3)),
+            sub(add(add(mul(a.e0, q.e1), mul(a.e1, q.e0)), mul(a.e2, q.e3)), mul(a.e3, q.e2)),
+            add(add(sub(mul(a.e0, q.e2), mul(a.e1, q.e3)), mul(a.e2, q.e0)), mul(a.e3, q.e1)),
+            add(sub(add(mul(a.e0, q.e3), mul(a.e1, q.e2)), mul(a.e2, q.e1)), mul(a.e3, q.e0))};
+}
+__device__ __forceinline__ Quat quat_angle_axis(double angle, double x, double y, double z) {   // QuatFromAngleAxis
+    const double h = mul(0.5, angle), s = sin(h);
+    return {cos(h), mul(x, s), mul(y, s), mul(z, s)};
+}
+// rotate_by: q <- normalize(QuatFromAngleAxis(|dth|, dth / |dth|) q)
+__device__ __forceinline__ Quat rotate_by(const Quat& q, double d0, double d1, double d2) {
+    const double a = sqrt(add(add(mul(d0, d0), mul(d1, d1)), mul(d2, d2)));
+    if (!(a > 0.0)) return q;
+    const double r = 1.0 / a;
+    Quat p = qmul(quat_angle_axis(a, mul(d0, r), mul(d1, r), mul(d2, r)), q);
+    const double n = sqrt(add(add(add(mul(p.e0, p.e0), mul(p.e1, p.e1)), mul(p.e2, p.e2)), mul(p.e3, p.e3)));
+    if (n > 0) { p.e0 = p.e0 / n; p.e1 = p.e1 / n; p.e2 = p.e2 / n; p.e3 = p.e3 / n; }
+    return p;
+}
+// GetCardanAnglesXYZ
+__device__ __forceinline__ void cardan_xyz(const Quat& q, double* out) {
+    const double r00 = sub(1.0, mul(2.0, add(mul(q.e2, q.e2), mul(q.e3, q.e3))));
+    const double r01 = mul(2.0, sub(mul(q.e1, q.e2), mul(q.e0, q.e3)));
+    const double r02 = mul(2.0, add(mul(q.e1, q.e3), mul(q.e0, q.e2)));
+    const double r12 = mul(2.0, sub(mul(q.e2, q.e3), mul(q.e0, q.e1)));
+    const double r22 = sub(1.0, mul(2.0, add(mul(q.e1, q.e1), mul(q.e2, q.e2))));
+    const double s = r02 > 1 ? 1 : (r02 < -1 ? -1 : r02);
+    out[0] = atan2(-r12, r22); out[1] = asin(s); out[2] = atan2(-r01, r00);
+}
+__device__ __forceinline__ Quat load_q(const double* p) { return {p[0], p[1], p[2], p[3]}; }
+__device__ __forceinline__ void store_q(double* p, const Quat& q) { p[0] = q.e0; p[1] = q.e1; p[2] = q.e2; p[3] = q.e3; }
+}  // namespace
+
+// One thread per instance.  The instance's generalised force lives in shared memory ([D][kBodyThreads], DoF-major so
+// that the lanes of a warp hit different banks); accelerations are sums over j = 0 .. D-1 in ascending order.
+__global__ void __launch_bounds__(kBodyThreads) k_body_step(const BodyStepArgs a, const int mode) {
+    extern __shared__ double s_F[];
+    const int b = blockIdx.x * kBodyThreads + threadIdx.x;
+    if (b >= a.B) return;
+    const int D = a.D;
+    const size_t o = (size_t)b * D;
+    double* F = s_F + threadIdx.x;
+    auto is_free = [&](int i) { return (a.free_mask >> i) & 1ull; };
+    constexpr double alpha = -0.2, gamma = 0.5 - alpha, beta = 0.25 * (1.0 - alpha) * (1.0 - alpha);
+
+    if (mode == kBodyInit) {
+        for (int n = 0; n < a.N; ++n) {
+            const double* x = a.pose_in + o + 6 * n;
+            Quat q;
+            double ang[3];
+            bool keep = false;
+            if (a.keep_q) {
+                q = load_q(a.q + ((size_t)b * a.N + n) * 4);
+                cardan_xyz(q, ang);
+                keep = ang[0] == x[3] && ang[1] == x[4] && ang[2] == x[5];
+            }
+            if (!keep) {      // QuatFromAngleX(roll) * QuatFromAngleY(pitch) * QuatFromAngleZ(yaw)
+                q = qmul(qmul(quat_angle_axis(x[3], 1, 0, 0), quat_angle_axis(x[4], 0, 1, 0)), quat_angle_axis(x[5], 0, 0, 1));
+                store_q(a.q + ((size_t)b * a.N + n) * 4, q);
+                cardan_xyz(q, ang);
+            }
+            for (int k = 0; k < 6; ++k) {
+                const double p = k < 3 ? x[k] : ang[k - 3], v = a.vel_in[o + 6 * n + k];
+                a.pose_out[o + 6 * n + k] = p; a.vel_out[o + 6 * n + k] = v;
+                if (a.sx) { a.sx[o + 6 * n + k] = p; a.sv[o + 6 * n + k] = v; }
+                if (a.x0) a.x0[o + 6 * n + k] = p;
+            }
+        }
+        return;
+    }
+
+    // generalised force at the evaluation state: hydro + gravity - PTO damper - PTO spring
+    for (int j = 0; j < D; ++j) {
+        double f = a.force[o + j];
+        const int k = j % 6;
+        if (k < 3) f = add(f, mul(a.mass[j / 6], a.g[k]));
+        const double v = a.vel_in[o + j];
+        if (a.pto_c) {
+            const double c = a.pto_c[o + j];
+            f = sub(f, mul(c, v));
+            if (a.energy && mode != kBodyHHTStart) a.energy[o + j] = add(a.energy[o + j], mul(mul(mul(c, v), v), a.dt));
+        }
+        if (a.pto_k) f = sub(f, mul(a.pto_k[o + j], sub(a.pose_in[o + j], a.x0[o + j])));
+        if (mode == kBodyHHTStep) {
+            const double fn = a.Fn[o + j];
+            a.Fn[o + j] = f;
+            f = sub(mul(1.0 + alpha, f), mul(alpha, fn));
+        } else if (mode == kBodyHHTStart) {
+            a.Fn[o + j] = f;
+        }
+        F[j * kBodyThreads] = f;
+    }
+    const double h = a.dt;
+    for (int n = 0; n < a.N; ++n) {
+        double acc[6];
+        for (int k = 0; k < 6; ++k) {
+            const double* row = a.Minv + (size_t)(6 * n + k) * D;
+            double s = 0.0;
+            for (int j = 0; j < D; ++j) s = add(s, mul(__ldg(row + j), F[j * kBodyThreads]));
+            acc[k] = s;
+        }
+        double* qp = a.q + ((size_t)b * a.N + n) * 4;
+        const size_t ob = o + 6 * n;
+        if (mode == kBodyEuler) {
+            double v[6];
+            for (int k = 0; k < 6; ++k) v[k] = is_free(6 * n + k) ? add(a.vel_in[ob + k], mul(h, acc[k])) : 0.0;
+            const Quat q = rotate_by(load_q(qp), mul(v[3], h), mul(v[4], h), mul(v[5], h));
+            store_q(qp, q);
+            double p[6];
+            for (int k = 0; k < 3; ++k) p[k] = add(a.pose_in[ob + k], mul(v[k], h));
+            cardan_xyz(q, p + 3);
+            for (int k = 0; k < 6; ++k) {
+                a.pose_out[ob + k] = p[k]; a.vel_out[ob + k] = v[k];
+                if (a.rec_pose) a.rec_pose[ob + k] = p[k];
+                if (a.rec_vel) a.rec_vel[ob + k] = v[k];
+            }
+            continue;
+        }
+        // HHT: corrector from the saved state x_n, v_n, q_n (kBodyHHTStart: acc are the initial accelerations)
+        double x[6], v[6], an[6];
+        for (int k = 0; k < 6; ++k) { x[k] = a.sx[ob + k]; v[k] = a.sv[ob + k]; }
+        Quat q = load_q(qp);
+        if (mode == kBodyHHTStep) {
+            double dth[3];
+            for (int k = 0; k < 6; ++k) {
+                const double a0 = a.an[ob + k], a1 = acc[k];
+                const double dv = mul(h, add(mul(1.0 - gamma, a0), mul(gamma, a1)));
+                const double dx = add(mul(h, v[k]), mul(mul(h, h), add(mul(0.5 - beta, a0), mul(beta, a1))));
+                if (k < 3) {
+                    if (is_free(6 * n + k)) { x[k] = add(x[k], dx); v[k] = add(v[k], dv); } else v[k] = 0.0;
+                } else {
+                    if (is_free(6 * n + k)) { dth[k - 3] = dx; v[k] = add(v[k], dv); } else { dth[k - 3] = 0.0; v[k] = 0.0; }
+                }
+            }
+            q = rotate_by(q, dth[0], dth[1], dth[2]);
+            store_q(qp, q);
+            cardan_xyz(q, x + 3);
+            for (int k = 0; k < 6; ++k) {
+                a.sx[ob + k] = x[k]; a.sv[ob + k] = v[k];
+                if (a.rec_pose) a.rec_pose[ob + k] = x[k];
+                if (a.rec_vel) a.rec_vel[ob + k] = v[k];
+            }
+        }
+        for (int k = 0; k < 6; ++k) { an[k] = acc[k]; a.an[ob + k] = acc[k]; }
+        // predictor of the next step: x* = x + h v + h^2/2 a,  v* = v + h a,  q* = rotate_by(q, h w + h^2/2 alpha)
+        const double hh2 = mul(mul(0.5, h), h);
+        double p[6], u[6];
+        for (int k = 0; k < 6; ++k) u[k] = add(v[k], mul(an[k], h));
+        for (int k = 0; k < 3; ++k) p[k] = add(add(x[k], mul(v[k], h)), mul(an[k], hh2));
+        const Quat qe = rotate_by(q, add(mul(v[3], h), mul(an[3], hh2)), add(mul(v[4], h), mul(an[4], hh2)),
+                                  add(mul(v[5], h), mul(an[5], hh2)));
+        store_q(a.qe + ((size_t)b * a.N + n) * 4, qe);
+        cardan_xyz(qe, p + 3);
+        for (int k = 0; k < 6; ++k) { a.pose_out[ob + k] = p[k]; a.vel_out[ob + k] = u[k]; }
+    }
+}
+
+cudaError_t launch_body_step(const BodyStepArgs& a, int mode, cudaStream_t st) {
+    const size_t smem = (size_t)a.D * kBodyThreads * sizeof(double);
+    k_body_step<<<(a.B + kBodyThreads - 1) / kBodyThreads, kBodyThreads, smem, st>>>(a, mode);
+    return cudaGetLastError();
+}
+
 }  // namespace hc

@@ -255,4 +255,42 @@ cudaError_t launch_lookahead(const LookaheadArgs& a, cudaStream_t st);
 cudaError_t launch_added_mass_mv(const double* M, int n_sys, int D, double c, const double* w, double* R, int B,
                                  cudaStream_t st);
 
+// ---- device-side stepping of free / ground-locked rigid bodies (hc_ensemble_simulate, k_body_step) ----
+// The force path evaluates the "evaluation state" (Euler: the state itself; HHT: the predictor); k_body_step reads it and
+// the step's hydro force and writes the next evaluation state into the other half of a ping-pong pair.
+enum BodyStepMode {
+    kBodyInit = 0,       // orientation from the caller's Cardan angles; evaluation state (+ HHT state, spring rest pose)
+    kBodyEuler = 1,      // linearised Euler step (ChSystem::StepEnd)
+    kBodyHHTStart = 2,   // HHT: initial accelerations from the force at t0, then the first predictor (StepHHTBegin)
+    kBodyHHTStep = 3     // HHT: corrector (StepHHTEnd), then the next predictor
+};
+constexpr int kBodyThreads = 64;
+struct BodyStepArgs {
+    const double* force;      // [B][D] hydro force of this step's evaluation (unused by kBodyInit)
+    const double* pose_in;    // [B][D] evaluation state (kBodyInit: the caller's initial state)
+    const double* vel_in;
+    double* pose_out;         // [B][D] next evaluation state
+    double* vel_out;
+    double* q;                // [B][N][4] orientation of the state
+    double* qe;               // [B][N][4] HHT: orientation of the predictor
+    double* sx;               // [B][D] HHT: state (positions, Cardan angles), updated in place
+    double* sv;               // [B][D] HHT: state velocities
+    double* Fn;               // [B][D] HHT: generalised force at t_n
+    double* an;               // [B][D] HHT: accelerations at t_n
+    double* x0;               // [B][D] spring rest pose (kBodyInit writes it when non-null)
+    const double* Minv;       // [D][D] inverse of the free-DoF mass matrix, zero rows / columns at locked DoFs
+    const double* pto_c;      // [B][D] or null
+    const double* pto_k;      // [B][D] or null
+    double* energy;           // [B][D] or null: += c v v dt with the evaluation velocity
+    double* rec_pose;         // [B][D] or null: state after this step
+    double* rec_vel;
+    double g[3];
+    double mass[kMaxBodies];
+    double dt;
+    unsigned long long free_mask;   // bit i: DoF i is free
+    int B, N, D;
+    int keep_q;               // kBodyInit: keep q of an instance whose Cardan angles equal the given ones bit for bit
+};
+cudaError_t launch_body_step(const BodyStepArgs& a, int mode, cudaStream_t st);
+
 }  // namespace hc

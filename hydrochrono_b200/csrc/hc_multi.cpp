@@ -230,6 +230,30 @@ hc_status hc_multi_waves_kinematics_at_time(hc_multi_ensemble* m, double t, int 
     });
 }
 
+hc_status hc_multi_ensemble_simulate(hc_multi_ensemble* m, const hc_sim_params* p, double* pose, double* vel, double* rec_t,
+                                     double* rec_pose, double* rec_vel, double* pto_energy, int* steps_done) {
+    if (steps_done) *steps_done = 0;
+    if (!p || !pose || !vel) { hc::set_last_error("null params, pose or vel"); return HC_ERR_INVALID; }
+    const size_t D = size_t(m->D), stride = size_t(m->B) * D;
+    std::atomic<int> fewest{p->n_steps};
+    const hc_status st = m->run([&](hc::Worker& k) {
+        const size_t off = size_t(k.first) * D;
+        hc_sim_params q = *p;
+        if (p->pto_damping) q.pto_damping = p->pto_damping + off;
+        if (p->pto_stiffness) q.pto_stiffness = p->pto_stiffness + off;
+        int done = 0;
+        // only the first shard writes the (shared) record times
+        const hc_status s = hc_ensemble_simulate_strided(k.ens, &q, pose + off, vel + off, k.first == 0 ? rec_t : nullptr,
+                                                         rec_pose ? rec_pose + off : nullptr, rec_vel ? rec_vel + off : nullptr,
+                                                         stride, pto_energy ? pto_energy + off : nullptr, &done);
+        int cur = fewest.load();
+        while (done < cur && !fewest.compare_exchange_weak(cur, done)) {}
+        return s;
+    });
+    if (steps_done) *steps_done = fewest.load();
+    return st;
+}
+
 hc_status hc_multi_get_components(hc_multi_ensemble* m, double* hs, double* rad, double* waves) {
     const int D = m->D;
     return m->run([=](hc::Worker& k) {

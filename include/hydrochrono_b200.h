@@ -282,6 +282,54 @@ HC_API hc_status hc_waves_kinematics_at_time(hc_ensemble* e, double t, int n_poi
 HC_API hc_status hc_waves_kinematics_at_time_device(hc_ensemble* e, double t, int n_points, const double* d_points,
                                                     double mwl, int wheeler_stretching,
                                                     double* d_eta, double* d_velocity, double* d_acceleration);
+/* ---- device-side stepping of the ensemble's bodies ----
+ * Advances every instance n_steps on the device: per step the force evaluation of hc_step_device, then one integrator
+ * kernel (k_body_step), no host synchronisation inside the loop.  Rigid bodies with 6 DoF each, every DoF free or locked
+ * to ground; forces = hydro + m g on translations + an optional linear PTO per instance and DoF,
+ * -k (x - x_init) - c v.  Mass matrix = diag(m, m, m, Ixx, Iyy, Izz) per body + the infinite-frequency added mass
+ * (hc_added_mass), restricted to the free DoFs, inverted once on the host per call.  Constrained multibody systems
+ * (joints between moving bodies, spring-damper geometry, contact) are not covered: step those with Chrono.
+ * The schemes follow the chrono_compat stepper (hydrochrono_b200/host/src/chrono_compat.cpp) operation for operation:
+ *   scheme 0, linearised Euler (ChSystem::StepEnd): forces at (t_n, x_n, v_n); v += dt a (locked DoFs: v = 0);
+ *     x += dt v; q <- normalize(QuatFromAngleAxis(|w dt|, w / |w|) q).
+ *   scheme 1, HHT-alpha with alpha = -0.2 (StepHHTBegin / StepHHTEnd): initial accelerations from the force at t0; the
+ *     force at t_{n+1} is evaluated at the predictor state (whose velocity enters the radiation history); the corrector
+ *     balances (1 + alpha) F_{n+1} - alpha F_n.  F_n and a_n stay on the device.  HHT evaluates n_steps + 1 forces.
+ * The device keeps one quaternion per body; the initial Cardan XYZ angles (roll, pitch, yaw) map to
+ * q = qx(roll) qy(pitch) qz(yaw), and the pose given to the force path and returned is (pos, GetCardanAnglesXYZ(q)).
+ * Times advance by repeated addition (t += dt), as Chrono advances ChTime.
+ * A second call with t0 equal to the previous end time continues the run: the orientation of a body whose given angles
+ * equal those of the ensemble's last quaternion bit for bit is kept, so Euler split into calls is bitwise identical to
+ * one call (without PTO springs, whose rest pose is each call's initial pose).  HHT restarts its acceleration history
+ * from the (time-cached) force at t0, as a freshly set-up ChSystem would.
+ * Arrays of hc_sim_params are host memory (copied at the call).  pto_energy = sum over the call's steps of
+ * c v_eval^2 dt per DoF, v_eval being the velocity of that step's force evaluation (the absorbed energy of a linear
+ * damper PTO; / (n_steps dt) gives the mean absorbed power).  Any output may be NULL.
+ * Errors of the force path (HC_ERR_ETA_WINDOW, HC_ERR_DUPLICATE_TIME, ...; all detected when a step is enqueued) end the
+ * run with that status: *steps_done = completed steps, pose / vel hold the state after the last completed step, the
+ * records and energy cover the completed steps.  HC_ERR_INVALID: n_steps < 1, record_every < 1, dt <= 0, mass or
+ * inertia NULL, pose or vel NULL, a singular free-DoF mass matrix. */
+typedef struct hc_sim_params {
+    int scheme;                 /* 0 = linearised Euler, 1 = HHT-alpha (alpha = -0.2) */
+    double t0, dt;
+    int n_steps, record_every;  /* record k = state after step (k+1)*record_every, k < n_steps / record_every */
+    double g[3];
+    const double* mass;         /* [N] */
+    const double* inertia;      /* [N][3], diagonal (ChBody::SetInertiaXX) */
+    const int* free_dof;        /* [6N] 1 free / 0 locked to ground; NULL = all free */
+    const double* pto_damping;  /* [B][6N] or NULL */
+    const double* pto_stiffness;/* [B][6N] or NULL; spring about the instance's initial pose */
+} hc_sim_params;
+/* Host buffers: pose / vel [B][6N] (in: initial state, out: final state), rec_t [n_rec], rec_pose / rec_vel
+ * [n_rec][B][6N], pto_energy [B][6N].  Records go through a device buffer of bounded size, copied out in chunks.
+ * Synchronous at return. */
+HC_API hc_status hc_ensemble_simulate(hc_ensemble* e, const hc_sim_params* p, double* pose, double* vel, double* rec_t,
+                                      double* rec_pose, double* rec_vel, double* pto_energy, int* steps_done);
+/* The same with pose, vel, rec_t, rec_pose, rec_vel and pto_energy as device pointers on the ensemble's device;
+ * asynchronous on the ensemble's stream (hc_sync waits). */
+HC_API hc_status hc_ensemble_simulate_device(hc_ensemble* e, const hc_sim_params* p, double* d_pose, double* d_vel,
+                                             double* d_rec_t, double* d_rec_pose, double* d_rec_vel, double* d_pto_energy,
+                                             int* steps_done);
 /* Re-stage the radiation kernel after hc_tables_set_convolution_mode() changed the ensemble's tables. */
 HC_API hc_status hc_ensemble_refresh_rirf(hc_ensemble* e);
 HC_API hc_status hc_sync(hc_ensemble* e);
@@ -396,6 +444,12 @@ HC_API hc_status hc_multi_step_device(hc_multi_ensemble* m, double t, const doub
 HC_API hc_status hc_multi_waves_kinematics_at_time(hc_multi_ensemble* m, double t, int n_points, const double* points,
                                                    double mwl, int wheeler_stretching,
                                                    double* eta, double* velocity, double* acceleration);
+/* hc_ensemble_simulate for every shard at once: host arrays in global instance order (pose / vel / pto_energy [B][6N],
+ * rec_pose / rec_vel [n_rec][B][6N], pto_* of the params [B][6N]).  Each shard runs its whole loop on its own worker
+ * thread, with no cross-shard barrier per step.  *steps_done = the fewest steps any shard completed. */
+HC_API hc_status hc_multi_ensemble_simulate(hc_multi_ensemble* m, const hc_sim_params* p, double* pose, double* vel,
+                                            double* rec_t, double* rec_pose, double* rec_vel, double* pto_energy,
+                                            int* steps_done);
 /* Final gather of the three force components of the last evaluation, host [B][6N] each (may be NULL). */
 HC_API hc_status hc_multi_get_components(hc_multi_ensemble* m, double* hydrostatic, double* radiation, double* waves);
 HC_API hc_status hc_multi_sync(hc_multi_ensemble* m);
