@@ -27,6 +27,49 @@ def sphere_raw():
             "bodies": [body]}
 
 
+def asymmetric_tables(raw, seed=11):
+    """Copy of raw tables whose matrices are not symmetric, so a row / column swap anywhere in a D x D path shows.
+    rirf_K: an independent factor 1 + 0.4 U(-1, 1) per (row, column), so the coupling blocks between bodies are
+    unrelated.  lin_matrix: every entry non-zero, off-diagonal terms small next to the diagonal (the stepping tests stay
+    stable).  inf_added_mass: 15 % of each entry's diagonal scale added per (row, column), the mass matrix stays well
+    conditioned.  Everything else is shared with raw."""
+    rng = np.random.Generator(np.random.MT19937(seed))
+    N = len(raw["bodies"])
+    D = 6 * N
+    fK = 1.0 + 0.4 * rng.uniform(-1.0, 1.0, size=(D, D))
+    A = np.concatenate([b["inf_added_mass"] for b in raw["bodies"]])
+    d = np.sqrt(np.abs(np.diag(A)))
+    A = A + 0.15 * np.outer(d, d) * rng.uniform(-1.0, 1.0, size=(D, D))
+    out = dict(raw, bodies=[])
+    for b, body in enumerate(raw["bodies"]):
+        Kh = np.asarray(body["lin_matrix"], dtype=np.float64)
+        scale = max(np.abs(np.diag(Kh)).max(), 1.0)
+        diag = np.where(np.diag(Kh) != 0.0, np.diag(Kh), 0.05 * scale * rng.uniform(0.5, 1.0, size=6))
+        off = 0.02 * np.sqrt(np.outer(np.abs(diag), np.abs(diag))) * rng.uniform(0.2, 1.0, size=(6, 6)) \
+            * rng.choice([-1.0, 1.0], size=(6, 6))
+        Kh = np.where(np.eye(6, dtype=bool), np.diag(diag), Kh + off)
+        nb = dict(body)
+        nb["rirf_K"] = np.asarray(body["rirf_K"]) * fK[6 * b:6 * b + 6, :, None]
+        nb["lin_matrix"] = Kh
+        nb["inf_added_mass"] = A[6 * b:6 * b + 6].copy()
+        out["bodies"].append(nb)
+    return out
+
+
+def transposed_tables(raw):
+    """raw with every matrix transposed: K per lag, each body's lin_matrix, the D x D infinite-frequency added mass."""
+    K = np.concatenate([b["rirf_K"] for b in raw["bodies"]]).transpose(1, 0, 2)
+    A = np.concatenate([b["inf_added_mass"] for b in raw["bodies"]]).T
+    out = dict(raw, bodies=[])
+    for b, body in enumerate(raw["bodies"]):
+        nb = dict(body)
+        nb["rirf_K"] = np.ascontiguousarray(K[6 * b:6 * b + 6])
+        nb["lin_matrix"] = np.ascontiguousarray(np.asarray(body["lin_matrix"]).T)
+        nb["inf_added_mass"] = np.ascontiguousarray(A[6 * b:6 * b + 6])
+        out["bodies"].append(nb)
+    return out
+
+
 def sphere_goldens():
     return np.load(os.path.join(GOLDEN, "sphere_goldens.npz"))
 

@@ -5,6 +5,7 @@ import math
 import numpy as np
 import pytest
 
+import common
 import hydrochrono_b200 as hc
 from hydrochrono_b200 import synth
 
@@ -105,7 +106,18 @@ def test_irregular_steps_are_rejected():
 def test_row_kernel_reproduces_the_reference_convolution(nb, steps, duration, dt):
     """sum_s K[:, :, s] w[s] lerp(v, t - t_s)  (hydro_forces.cpp:586-647)  ==  sum_i Krow[i] v[row i]  for a history on a
     uniform grid: the row-grid kernel folds the interpolation weights in, the lag-grid kernel is (K w) itself."""
-    raw = synth.make_tables(num_bodies=nb, rirf_steps=steps, rirf_duration=duration)
+    _check_row_kernel(synth.make_tables(num_bodies=nb, rirf_steps=steps, rirf_duration=duration), nb, steps, duration, dt)
+
+
+@pytest.mark.parametrize("nb,steps,duration,dt", [(2, 601, 30.0, 0.03), (1, 401, 4.0, 0.01), (2, 1001, 60.0, 0.01)])
+def test_row_kernel_reproduces_the_reference_convolution_asymmetric(nb, steps, duration, dt):
+    """The same identity with non-symmetric K (common.asymmetric_tables): on symmetric K a row kernel applied
+    transposed would pass it."""
+    raw = common.asymmetric_tables(synth.make_tables(num_bodies=nb, rirf_steps=steps, rirf_duration=duration))
+    _check_row_kernel(raw, nb, steps, duration, dt)
+
+
+def _check_row_kernel(raw, nb, steps, duration, dt):
     T = hc.Tables.from_raw(raw)
     D = 6 * nb
     mode, m, lk = T.rad_lookahead_plan(dt)
@@ -144,7 +156,19 @@ def test_block_decomposition_is_the_full_convolution(nb, steps, duration, dt, ba
     library's own row kernel: for a block whose snapshot of the history was taken `base` steps before its first step,
         F_j = sum_u Krow[u + g + 1] v_res[m u + m - 1 - rho]  +  sum_{l <= jj / m} Krow[l] v_young[jj - m l],
     jj = base + j = rho + m g, equals the convolution of all rows with the row kernel."""
-    raw = synth.make_tables(num_bodies=nb, rirf_steps=steps, rirf_duration=duration)
+    _check_block_decomposition(synth.make_tables(num_bodies=nb, rirf_steps=steps, rirf_duration=duration), nb, dt,
+                               base_blocks)
+
+
+@pytest.mark.parametrize("nb,steps,duration,dt", [(2, 1001, 60.0, 0.01), (2, 601, 30.0, 0.03)])
+@pytest.mark.parametrize("base_blocks", [0, 1])
+def test_block_decomposition_is_the_full_convolution_asymmetric(nb, steps, duration, dt, base_blocks):
+    """The same identity with non-symmetric K (common.asymmetric_tables)."""
+    raw = common.asymmetric_tables(synth.make_tables(num_bodies=nb, rirf_steps=steps, rirf_duration=duration))
+    _check_block_decomposition(raw, nb, dt, base_blocks)
+
+
+def _check_block_decomposition(raw, nb, dt, base_blocks):
     T = hc.Tables.from_raw(raw)
     D = 6 * nb
     mode, m, lk = T.rad_lookahead_plan(dt)
