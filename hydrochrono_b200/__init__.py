@@ -572,6 +572,12 @@ class Ensemble:
         _check(lib.hc_get_rad_block_stats(self._h, C.byref(n), C.byref(served), C.byref(ms), int(reset)))
         return {"launches": n.value, "steps_served": served.value, "avg_ms": ms.value}
 
+    def exc_block_stats(self, reset=True):
+        """Excitation look-ahead: blocks built and steps whose wave force came from a block (hc_get_exc_block_stats)."""
+        n, served = C.c_longlong(), C.c_longlong()
+        _check(lib.hc_get_exc_block_stats(self._h, C.byref(n), C.byref(served), int(reset)))
+        return {"blocks": n.value, "steps_served": served.value}
+
     def close(self):
         if getattr(self, "_h", None):
             lib.hc_ensemble_destroy(self._h)

@@ -139,6 +139,7 @@ SIGNATURES = {
     "hc_rad_lookahead_check_step": (C.c_int, [vp, C.c_double, C.c_double, dp, C.c_int, C.POINTER(C.c_int)]),
     "hc_ensemble_rad_lookahead_steps": (C.c_int, [vp]),
     "hc_get_rad_block_stats": (C.c_int, [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong), dp, C.c_int]),
+    "hc_get_exc_block_stats": (C.c_int, [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong), C.c_int]),
     "hc_multi_shard_range": (None, [C.c_int, C.c_int, C.c_int, ip, ip]),
     "hc_multi_ensemble_create": (C.c_int, [vp, C.POINTER(EnsembleOpts), ip, C.c_int, C.POINTER(vp)]),
     "hc_multi_ensemble_destroy": (None, [vp]),

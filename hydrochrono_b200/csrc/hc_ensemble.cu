@@ -248,6 +248,7 @@ struct hc_ensemble {
     cudaEvent_t ev_la_done[2] = {nullptr, nullptr}, ev_la_free[2] = {nullptr, nullptr}, ev_la_build = nullptr;
     cudaEvent_t ev_la_join = nullptr;
     int la_builds = 0, la_hits_this_block = 0, la_poor_blocks = 0;
+    long long la_blocks_built = 0, la_steps_served = 0;   // hc_get_exc_block_stats (never cleared by a reset)
     DevBuf<double> d_la_cache, d_la_times;
     cudaEvent_t ev_la[2] = {nullptr, nullptr};
     bool la_events_pending = false;
@@ -1062,7 +1063,7 @@ int hc_ensemble::enqueue_lookahead_block(int buf, double t0, cudaStream_t st, in
     if (timed) { CUDA_CHECK(cudaEventRecord(ev_la[1], st)); la_events_pending = true; }
     CUDA_CHECK(cudaEventRecord(ev_la_build, st));
     Bk.len = T; Bk.valid = true;
-    ++la_builds;
+    ++la_builds; ++la_blocks_built;
     return T;
 }
 
@@ -1096,7 +1097,7 @@ int hc_ensemble::lookahead_slot(double t) {
     LaBlock& Cur = la_blk[la_cur];
     if (Cur.valid && la_pos < Cur.len && Cur.times[la_pos] == t) {
         if (la_pos >= kLaT / 2) finish_split_build();
-        ++la_hits_this_block;
+        ++la_hits_this_block; ++la_steps_served;
         return la_cur * kLaT + la_pos++;
     }
     finish_split_build();             // a switch or a rebuild follows: the build in flight must be complete (its scratch
@@ -1108,6 +1109,7 @@ int hc_ensemble::lookahead_slot(double t) {
         CUDA_CHECK(cudaStreamWaitEvent(stream, ev_la_done[la_cur], 0));
         CUDA_CHECK(cudaEventRecord(ev_la_free[old], stream));     // every reader of `old` is already enqueued
         prefetch_lookahead(old);
+        ++la_steps_served;
         return la_cur * kLaT + la_pos++;
     }
     // miss: first step, end of a block without prefetch, or a time the prediction did not foresee
@@ -1122,7 +1124,7 @@ int hc_ensemble::lookahead_slot(double t) {
         CUDA_CHECK(cudaEventRecord(ev_la_free[la_cur ^ 1], stream));
         prefetch_lookahead(la_cur ^ 1);
     }
-    ++la_hits_this_block;
+    ++la_hits_this_block; ++la_steps_served;
     return la_cur * kLaT + la_pos++;
 }
 
@@ -1322,6 +1324,8 @@ hc_status hc_ensemble_reset(hc_ensemble* e) {
     e->last_step_fast = false;
     e->prev_time = -1.0;
     e->force_valid = false;
+    // a new run builds its orientations from the given angles, as a fresh ensemble does: no quaternion is kept
+    e->sim_q_valid = false;
     CUDA_CHECK(cudaMemsetAsync(e->d_force.p, 0, e->d_force.n * sizeof(double), e->stream));
     CUDA_CHECK(cudaMemsetAsync(e->d_comp.p, 0, e->d_comp.n * sizeof(double), e->stream));
     return HC_OK;
@@ -2296,6 +2300,13 @@ hc_status hc_get_rad_block_stats(hc_ensemble* e, long long* launches, long long*
     if (reset) { e->rb_launches = 0; e->rb_steps_served = 0; e->rb_items_timed = 0; e->rb_ms_sum = 0.0; }
     return HC_OK;
     HC_GUARD_END
+}
+
+hc_status hc_get_exc_block_stats(hc_ensemble* e, long long* blocks_built, long long* steps_served, int reset) {
+    if (blocks_built) *blocks_built = e->la_blocks_built;
+    if (steps_served) *steps_served = e->la_steps_served;
+    if (reset) { e->la_blocks_built = 0; e->la_steps_served = 0; }
+    return HC_OK;
 }
 
 hc_status hc_measure_fp64_mma_peak(int device, double* tflops) {

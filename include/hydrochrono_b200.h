@@ -185,7 +185,8 @@ HC_API hc_status hc_ensemble_create(const hc_tables* t, const hc_ensemble_opts* 
 HC_API void hc_ensemble_destroy(hc_ensemble* e);
 HC_API int hc_ensemble_batch(const hc_ensemble* e);
 HC_API int hc_ensemble_dofs(const hc_ensemble* e);      /* 6N */
-/* Drops the velocity history and the time cache (a fresh TestHydro), keeps the waves. */
+/* Drops the velocity history, the time cache and the orientations kept by hc_ensemble_simulate (a fresh TestHydro),
+ * keeps the waves. */
 HC_API hc_status hc_ensemble_reset(hc_ensemble* e);
 /* Changes hc_ensemble_opts.bracket_snap for the following steps (0 = bit-faithful bracketing). */
 HC_API hc_status hc_ensemble_set_bracket_snap(hc_ensemble* e, double snap);
@@ -300,8 +301,9 @@ HC_API hc_status hc_waves_kinematics_at_time_device(hc_ensemble* e, double t, in
  * Times advance by repeated addition (t += dt), as Chrono advances ChTime.
  * A second call with t0 equal to the previous end time continues the run: the orientation of a body whose given angles
  * equal those of the ensemble's last quaternion bit for bit is kept, so Euler split into calls is bitwise identical to
- * one call (without PTO springs, whose rest pose is each call's initial pose).  HHT restarts its acceleration history
- * from the (time-cached) force at t0, as a freshly set-up ChSystem would.
+ * one call (without PTO springs, whose rest pose is each call's initial pose).  The rule applies only to such a
+ * continuation: after hc_ensemble_reset every orientation is built from the given angles, as in a fresh ensemble.
+ * HHT restarts its acceleration history from the (time-cached) force at t0, as a freshly set-up ChSystem would.
  * Arrays of hc_sim_params are host memory (copied at the call).  pto_energy = sum over the call's steps of
  * c v_eval^2 dt per DoF, v_eval being the velocity of that step's force evaluation (the absorbed energy of a linear
  * damper PTO; / (n_steps dt) gives the mean absorbed power).  Any output may be NULL.
@@ -373,6 +375,9 @@ HC_API hc_status hc_get_kernel_ms(hc_ensemble* e, double* prestep_ms, double* ra
 HC_API int hc_ensemble_rad_lookahead_steps(const hc_ensemble* e);
 HC_API hc_status hc_get_rad_block_stats(hc_ensemble* e, long long* launches, long long* steps_served, double* avg_ms,
                                         int reset);
+/* Excitation look-ahead (hc_ensemble_opts.exc_lookahead): blocks of wave forces built so far (a split build counts
+   once) and how many steps took their wave force from a block instead of the per-step excitation kernels. */
+HC_API hc_status hc_get_exc_block_stats(hc_ensemble* e, long long* blocks_built, long long* steps_served, int reset);
 
 /* Host-side planning of the radiation look-ahead, exposed for testing (no device needed).
    hc_rad_lookahead_plan: mode = 0 (the look-ahead cannot serve this step size), 1 (lag grid: RIRF lag spacing =
