@@ -11,7 +11,7 @@ import numpy as np
 from . import _capi
 from ._capi import lib
 
-__all__ = ["Tables", "Ensemble", "HydroError", "DuplicateTimeError", "EtaWindowError", "version", "device_count"]
+__all__ = ["Tables", "Ensemble", "Prismatic", "TSDA", "HydroError", "DuplicateTimeError", "EtaWindowError", "version", "device_count"]
 
 
 class HydroError(RuntimeError):
@@ -131,8 +131,68 @@ def _ptr(x):
 _SCHEMES = {"euler": 0, "hht": 1, 0: 0, 1: 1}
 
 
+class Prismatic:
+    """ChLinkLockPrismatic for device stepping: body `child` keeps one slide DoF along `axis` (world frame at
+    assembly) relative to body `parent` (-1: ground)."""
+
+    def __init__(self, child, parent, axis=(0.0, 0.0, 1.0)):
+        self.child, self.parent = int(child), int(parent)
+        self.axis = tuple(float(v) for v in axis)
+
+    def __repr__(self):
+        return "Prismatic(%d, %d, %r)" % (self.child, self.parent, self.axis)
+
+
+class TSDA:
+    """ChLinkTSDA for device stepping: spring-damper between point1 on body1 and point2 on body2 (world frame at
+    assembly; body index -1: ground).  damping / stiffness: scalar or one value per instance [B]; rest_length None =
+    the length at assembly."""
+
+    def __init__(self, body1, body2, point1, point2, damping=0.0, stiffness=0.0, rest_length=None):
+        self.body1, self.body2 = int(body1), int(body2)
+        self.point1 = tuple(float(v) for v in point1)
+        self.point2 = tuple(float(v) for v in point2)
+        self.damping, self.stiffness, self.rest_length = damping, stiffness, rest_length
+
+    def __repr__(self):
+        return "TSDA(%d, %d, %r, %r, damping=%r, stiffness=%r, rest_length=%r)" % (
+            self.body1, self.body2, self.point1, self.point2, self.damping, self.stiffness, self.rest_length)
+
+
+def _sim_links(batch, prismatic, tsda, keep):
+    """hc_sim_links for the given joints / spring-dampers (None when there are none); arrays kept alive in `keep`."""
+    prismatic, tsda = list(prismatic or []), list(tsda or [])
+    if not prismatic and not tsda:
+        return None
+    L = _capi.SimLinks()
+    L.n_prismatic, L.n_tsda = len(prismatic), len(tsda)
+    if prismatic:
+        arr = (_capi.SimPrismatic * len(prismatic))()
+        for i, j in enumerate(prismatic):
+            arr[i].child, arr[i].parent = j.child, j.parent
+            for k in range(3):
+                arr[i].axis[k] = j.axis[k]
+        keep["prismatic"] = arr
+        L.prismatic = C.cast(arr, C.POINTER(_capi.SimPrismatic))
+    if tsda:
+        arr = (_capi.SimTSDA * len(tsda))()
+        for i, s in enumerate(tsda):
+            arr[i].body1, arr[i].body2 = s.body1, s.body2
+            for k in range(3):
+                arr[i].point1[k], arr[i].point2[k] = s.point1[k], s.point2[k]
+            arr[i].rest_length = -1.0 if s.rest_length is None else float(s.rest_length)
+        keep["tsda"] = arr
+        L.tsda = C.cast(arr, C.POINTER(_capi.SimTSDA))
+        for name, attr in (("tsda_c", "damping"), ("tsda_k", "stiffness")):
+            cols = [np.broadcast_to(np.asarray(getattr(s, attr), dtype=np.float64), (batch,)) for s in tsda]
+            keep[name] = _f64(np.stack(cols, axis=1))
+        L.tsda_damping, L.tsda_stiffness = _dp(keep["tsda_c"]), _dp(keep["tsda_k"])
+    keep["links"] = L
+    return L
+
+
 def _sim_params(dofs, batch, n_steps, dt, t0, scheme, record_every, gvec, mass, inertia, free_dof, pto_damping,
-                pto_stiffness):
+                pto_stiffness, prismatic=None, tsda=None):
     """hc_sim_params and the arrays it points to (kept alive by the caller through the returned tuple)."""
     if scheme not in _SCHEMES:
         raise ValueError("scheme must be 'euler' or 'hht'")
@@ -151,29 +211,37 @@ def _sim_params(dofs, batch, n_steps, dt, t0, scheme, record_every, gvec, mass, 
     p.mass, p.inertia = _dp(keep["mass"]), _dp(keep["inertia"])
     p.free_dof = keep["free"].ctypes.data_as(_capi.ip) if "free" in keep else None
     p.pto_damping, p.pto_stiffness = _dp(keep.get("c")), _dp(keep.get("k"))
+    L = _sim_links(batch, prismatic, tsda, keep)
+    p.links = C.pointer(L) if L is not None else None
     return p, keep
 
 
-def _simulate_host(fn, handle, batch, dofs, pose0, vel0, n_steps, record_every, record, energy, p):
+def _simulate_host(fn, handle, batch, dofs, pose0, vel0, n_steps, record_every, record, energy, p, keep):
     pose = _f64(pose0).reshape(batch, dofs).copy()
     vel = np.zeros((batch, dofs)) if vel0 is None else _f64(vel0).reshape(batch, dofs).copy()
     n_rec = n_steps // max(int(record_every), 1) if record else 0
     times, rp, rv = np.empty(n_rec), np.empty((n_rec, batch, dofs)), np.empty((n_rec, batch, dofs))
     e = np.empty((batch, dofs)) if energy else None
+    te = None
+    L = keep.get("links")
+    if L is not None and L.n_tsda > 0 and energy:
+        te = np.empty((batch, L.n_tsda))
+        L.tsda_energy = te.ctypes.data
     done = C.c_int()
     st = fn(handle, C.byref(p), _dp(pose), _dp(vel), _dp(times) if n_rec else None, _dp(rp) if n_rec else None,
             _dp(rv) if n_rec else None, _dp(e), C.byref(done))
-    return st, SimResult(times, rp, rv, e, done.value, pose, vel)
+    return st, SimResult(times, rp, rv, e, done.value, pose, vel, te)
 
 
 class SimResult(tuple):
     """(times, pose, vel, pto_energy, steps_done) of a device-stepped run: times [n_rec] and pose / vel
     [n_rec][B][6N] are the recorded states (state after step (k+1) record_every), pto_energy [B][6N] (or None);
-    final_pose / final_vel [B][6N] are the state after the last completed step."""
+    final_pose / final_vel [B][6N] are the state after the last completed step; tsda_energy [B][n_tsda] is the energy
+    each spring-damper absorbed, sum c ldot^2 dt (None without spring-dampers or with energy=False)."""
 
-    def __new__(cls, times, pose, vel, energy, steps_done, final_pose, final_vel):
+    def __new__(cls, times, pose, vel, energy, steps_done, final_pose, final_vel, tsda_energy=None):
         r = super().__new__(cls, (times, pose, vel, energy, steps_done))
-        r.final_pose, r.final_vel = final_pose, final_vel
+        r.final_pose, r.final_vel, r.tsda_energy = final_pose, final_vel, tsda_energy
         return r
 
 
@@ -488,16 +556,18 @@ class Ensemble:
 
     def simulate(self, pose0, n_steps, dt, mass, inertia, vel0=None, t0=0.0, scheme="euler", record_every=1,
                  gvec=(0.0, 0.0, -9.81), free_dof=None, pto_damping=None, pto_stiffness=None, record=True,
-                 energy=True, check=True):
+                 energy=True, check=True, prismatic=None, tsda=None):
         """Advances every instance n_steps on the device (hc_ensemble_simulate): rigid bodies with each DoF free or
         locked to ground (free_dof [6N], None = all free), gravity, optional linear PTO per instance and DoF
         (pto_damping / pto_stiffness [B][6N] or broadcastable).  scheme 'euler' (linearised Euler) or 'hht'
-        (HHT-alpha, alpha = -0.2).  Returns SimResult (times, pose, vel, pto_energy, steps_done) as numpy arrays;
+        (HHT-alpha, alpha = -0.2).  prismatic / tsda: lists of Prismatic joints and TSDA spring-dampers (the RM3
+        float on its spar with a PTO), stepped in reduced coordinates on the device (k_body_step_linked).  Returns
+        SimResult (times, pose, vel, pto_energy, steps_done) as numpy arrays, with result.tsda_energy [B][n_tsda];
         with check=False a force-path error is returned as result.status instead of raised."""
         p, keep = _sim_params(self.dofs, self.batch, n_steps, dt, t0, scheme, record_every, gvec, mass, inertia,
-                              free_dof, pto_damping, pto_stiffness)
+                              free_dof, pto_damping, pto_stiffness, prismatic, tsda)
         st, res = _simulate_host(lib.hc_ensemble_simulate, self._h, self.batch, self.dofs, pose0, vel0, n_steps,
-                                 record_every, record, energy, p)
+                                 record_every, record, energy, p, keep)
         res.status = st
         if check:
             _check(st)
@@ -505,12 +575,16 @@ class Ensemble:
 
     def simulate_device(self, d_pose, d_vel, n_steps, dt, mass, inertia, t0=0.0, scheme="euler", record_every=1,
                         gvec=(0.0, 0.0, -9.81), free_dof=None, pto_damping=None, pto_stiffness=None, d_rec_t=None,
-                        d_rec_pose=None, d_rec_vel=None, d_pto_energy=None):
+                        d_rec_pose=None, d_rec_vel=None, d_pto_energy=None, prismatic=None, tsda=None,
+                        d_tsda_energy=None):
         """simulate on device buffers (torch CUDA tensors or raw addresses): d_pose / d_vel [B][6N] in: initial
-        state, out: final state; d_rec_t [n_rec], d_rec_pose / d_rec_vel [n_rec][B][6N], d_pto_energy [B][6N], any
-        may be None.  Asynchronous on the ensemble stream.  Returns steps_done (force-path errors are raised)."""
+        state, out: final state; d_rec_t [n_rec], d_rec_pose / d_rec_vel [n_rec][B][6N], d_pto_energy [B][6N],
+        d_tsda_energy [B][n_tsda], any may be None.  Asynchronous on the ensemble stream.  Returns steps_done
+        (force-path errors are raised)."""
         p, keep = _sim_params(self.dofs, self.batch, n_steps, dt, t0, scheme, record_every, gvec, mass, inertia,
-                              free_dof, pto_damping, pto_stiffness)
+                              free_dof, pto_damping, pto_stiffness, prismatic, tsda)
+        if keep.get("links") is not None and d_tsda_energy is not None:
+            keep["links"].tsda_energy = _ptr(d_tsda_energy).value
         done = C.c_int()
         _check(lib.hc_ensemble_simulate_device(self._h, C.byref(p), _ptr(d_pose), _ptr(d_vel), _ptr(d_rec_t),
                                                _ptr(d_rec_pose), _ptr(d_rec_vel), _ptr(d_pto_energy), C.byref(done)))
@@ -682,13 +756,13 @@ class MultiEnsemble:
 
     def simulate(self, pose0, n_steps, dt, mass, inertia, vel0=None, t0=0.0, scheme="euler", record_every=1,
                  gvec=(0.0, 0.0, -9.81), free_dof=None, pto_damping=None, pto_stiffness=None, record=True,
-                 energy=True, check=True):
+                 energy=True, check=True, prismatic=None, tsda=None):
         """Ensemble.simulate over every shard (hc_multi_ensemble_simulate), arrays in global instance order; each
         shard runs its whole loop on its own worker thread."""
         p, keep = _sim_params(self.dofs, self.batch, n_steps, dt, t0, scheme, record_every, gvec, mass, inertia,
-                              free_dof, pto_damping, pto_stiffness)
+                              free_dof, pto_damping, pto_stiffness, prismatic, tsda)
         st, res = _simulate_host(lib.hc_multi_ensemble_simulate, self._h, self.batch, self.dofs, pose0, vel0, n_steps,
-                                 record_every, record, energy, p)
+                                 record_every, record, energy, p, keep)
         res.status = st
         if check:
             _check(st)

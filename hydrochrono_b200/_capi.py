@@ -57,10 +57,24 @@ class ProfileStats(C.Structure):
                 ("eta_synthesis_seconds", C.c_double), ("step_seconds", C.c_double), ("kernel_launches", C.c_longlong)]
 
 
+class SimPrismatic(C.Structure):
+    _fields_ = [("child", C.c_int), ("parent", C.c_int), ("axis", C.c_double * 3)]
+
+
+class SimTSDA(C.Structure):
+    _fields_ = [("body1", C.c_int), ("body2", C.c_int), ("point1", C.c_double * 3), ("point2", C.c_double * 3),
+                ("rest_length", C.c_double)]
+
+
+class SimLinks(C.Structure):
+    _fields_ = [("n_prismatic", C.c_int), ("n_tsda", C.c_int), ("prismatic", C.POINTER(SimPrismatic)),
+                ("tsda", C.POINTER(SimTSDA)), ("tsda_damping", dp), ("tsda_stiffness", dp), ("tsda_energy", vp)]
+
+
 class SimParams(C.Structure):
     _fields_ = [("scheme", C.c_int), ("t0", C.c_double), ("dt", C.c_double), ("n_steps", C.c_int),
                 ("record_every", C.c_int), ("g", C.c_double * 3), ("mass", dp), ("inertia", dp), ("free_dof", ip),
-                ("pto_damping", dp), ("pto_stiffness", dp)]
+                ("pto_damping", dp), ("pto_stiffness", dp), ("links", C.POINTER(SimLinks))]
 
 
 # every symbol include/hydrochrono_b200.h declares: name -> (restype, argtypes)

@@ -192,6 +192,11 @@ struct hc_ensemble {
     size_t h_rec_bytes = 0;
     bool sim_q_valid = false;                     // d_simq holds the orientations of the last run's final state
     double* sim(int slot) { return d_sim.p + size_t(slot) * B * D; }
+    // runs with joints / spring-dampers (k_body_step_linked): full mass matrix, per-instance assembly data, the pose the
+    // last linked run ended in (continuation test), spring-damper coefficients [2][B][n_tsda] and the host variant's energy
+    DevBuf<double> d_link_M, d_link_asm, d_link_end, d_link_coef, d_link_energy;
+    bool link_asm_valid = false;                  // d_link_asm / d_link_end belong to the last run, which had links link_key
+    std::vector<double> link_key;
 
     // waves
     int wave_mode = 0;
@@ -1326,6 +1331,7 @@ hc_status hc_ensemble_reset(hc_ensemble* e) {
     e->force_valid = false;
     // a new run builds its orientations from the given angles, as a fresh ensemble does: no quaternion is kept
     e->sim_q_valid = false;
+    e->link_asm_valid = false;                    // ... and every joint / spring-damper is assembled again
     CUDA_CHECK(cudaMemsetAsync(e->d_force.p, 0, e->d_force.n * sizeof(double), e->stream));
     CUDA_CHECK(cudaMemsetAsync(e->d_comp.p, 0, e->d_comp.n * sizeof(double), e->stream));
     return HC_OK;
@@ -2007,6 +2013,87 @@ static std::vector<double> sim_inverse_mass(const hc_tables* T, const hc_sim_par
     return Minv;
 }
 
+// Validation and descriptors of a run with joints / spring-dampers (k_body_step_linked): fills the link fields of la,
+// the full mass matrix M = diag(m, m, m, Ixx, Iyy, Izz) + A_inf and the key that identifies the links (continuation).
+static void sim_links_setup(const hc_tables* T, const hc_sim_params& p, unsigned long long free_mask, LinkStepArgs& la,
+                            std::vector<double>& M, std::vector<double>& key) {
+    const hc_sim_links& L = *p.links;
+    const int N = T->N, D = T->D;
+    auto bad = [](const std::string& m) { fail(HC_ERR_INVALID, "hc_ensemble_simulate: " + m); };
+    if (L.n_prismatic < 0 || L.n_tsda < 0) bad("negative joint or spring-damper count");
+    if ((L.n_prismatic > 0 && !L.prismatic) || (L.n_tsda > 0 && !L.tsda)) bad("null joint or spring-damper array");
+    if (L.n_tsda > kMaxLinkTsda) bad("more than " + std::to_string(kMaxLinkTsda) + " spring-dampers");
+    if (L.n_prismatic > N) bad("more joints than bodies (a body is the child of one joint at most)");
+    for (int n = 0; n < kMaxBodies; ++n) { la.parent_of[n] = -2; la.joint_of[n] = -1; }
+    for (int j = 0; j < L.n_prismatic; ++j) {
+        const hc_sim_prismatic& J = L.prismatic[j];
+        if (J.child < 0 || J.child >= N || J.parent < -1 || J.parent >= N) bad("joint body index out of range");
+        if (J.child == J.parent) bad("joint child == parent");
+        if (la.joint_of[J.child] >= 0) bad("a second joint on one child");
+        const double n2 = J.axis[0] * J.axis[0] + J.axis[1] * J.axis[1] + J.axis[2] * J.axis[2];
+        if (!(n2 > 0.0) || !std::isfinite(n2)) bad("zero or non-finite joint axis");
+        const double n = std::sqrt(n2);
+        la.joint_of[J.child] = j;
+        la.parent_of[J.child] = J.parent;
+        la.pr_child[j] = J.child; la.pr_parent[j] = J.parent;
+        for (int k = 0; k < 3; ++k) la.pr_axis[j][k] = J.axis[k] / n;
+        for (int k = 0; k < 6; ++k)
+            if (!((free_mask >> (6 * J.child + k)) & 1ull)) bad("a jointed child must have every DoF free");
+    }
+    for (int j = 0; j < L.n_prismatic; ++j)
+        if (la.pr_parent[j] >= 0 && la.joint_of[la.pr_parent[j]] >= 0) bad("chains of joints are not supported");
+    for (int t = 0; t < L.n_tsda; ++t) {
+        const hc_sim_tsda& S = L.tsda[t];
+        if (S.body1 < -1 || S.body1 >= N || S.body2 < -1 || S.body2 >= N) bad("spring-damper body index out of range");
+        if (S.body1 == S.body2) bad(S.body1 < 0 ? "spring-damper between ground and ground" : "spring-damper body1 == body2");
+        la.ts_b1[t] = S.body1; la.ts_b2[t] = S.body2; la.ts_rest[t] = S.rest_length;
+        for (int k = 0; k < 3; ++k) { la.ts_p1[t][k] = S.point1[k]; la.ts_p2[t][k] = S.point2[k]; }
+    }
+    la.n_pr = L.n_prismatic; la.n_tsda = L.n_tsda;
+    // columns of T: the free DoFs of every root body in body order, then one slide per child in body order
+    int nq = 0;
+    for (int n = 0; n < N; ++n)
+        if (la.joint_of[n] < 0)
+            for (int k = 0; k < 6; ++k)
+                if ((free_mask >> (6 * n + k)) & 1ull) { la.col_body[nq] = (signed char)n; la.col_dof[nq] = (signed char)k; ++nq; }
+    for (int n = 0; n < N; ++n)
+        if (la.joint_of[n] >= 0) { la.col_body[nq] = (signed char)n; la.col_dof[nq] = 6; ++nq; }
+    la.nq = nq;
+    M.assign(size_t(D) * D, 0.0);
+    for (int i = 0; i < D; ++i) {
+        const int b = i / 6, k = i % 6;
+        M[size_t(i) * D + i] = k < 3 ? p.mass[b] : p.inertia[3 * b + k - 3];
+    }
+    for (int i = 0; i < D; ++i)
+        for (int j = 0; j < D; ++j) M[size_t(i) * D + j] += T->body[i / 6].ainf[size_t(i % 6) * D + j];
+    // Cholesky of the symmetric part: positive definite => T^T M T is nonsingular for every full-column-rank T
+    std::vector<double> C(size_t(D) * D);
+    for (int i = 0; i < D; ++i)
+        for (int j = 0; j < D; ++j) C[size_t(i) * D + j] = 0.5 * (M[size_t(i) * D + j] + M[size_t(j) * D + i]);
+    for (int j = 0; j < D; ++j) {
+        double d = C[size_t(j) * D + j];
+        for (int k = 0; k < j; ++k) d -= C[size_t(j) * D + k] * C[size_t(j) * D + k];
+        if (!(d > 0.0) || !std::isfinite(d)) bad("the mass matrix diag(m, I) + A_inf is not positive definite");
+        const double r = std::sqrt(d);
+        C[size_t(j) * D + j] = r;
+        for (int i = j + 1; i < D; ++i) {
+            double s = C[size_t(i) * D + j];
+            for (int k = 0; k < j; ++k) s -= C[size_t(i) * D + k] * C[size_t(j) * D + k];
+            C[size_t(i) * D + j] = s / r;
+        }
+    }
+    key.clear();
+    for (int j = 0; j < la.n_pr; ++j) {
+        key.push_back(la.pr_child[j]); key.push_back(la.pr_parent[j]);
+        for (int k = 0; k < 3; ++k) key.push_back(la.pr_axis[j][k]);
+    }
+    key.push_back(-1.0);
+    for (int t = 0; t < la.n_tsda; ++t) {
+        key.push_back(la.ts_b1[t]); key.push_back(la.ts_b2[t]); key.push_back(la.ts_rest[t]);
+        for (int k = 0; k < 3; ++k) { key.push_back(la.ts_p1[t][k]); key.push_back(la.ts_p2[t][k]); }
+    }
+}
+
 // host = true: pose, vel, rec_*, energy are host memory (records through a bounded device buffer, copied out in chunks;
 // record k of rec_pose / rec_vel starts at element k * rec_stride).  host = false: device memory, rec_stride = B D.
 static hc_status sim_run(hc_ensemble* e, const hc_sim_params* p, bool host, double* pose, double* vel, double* rec_t,
@@ -2023,13 +2110,43 @@ static hc_status sim_run(hc_ensemble* e, const hc_sim_params* p, bool host, doub
     const size_t bd = size_t(B) * D, bytes = bd * sizeof(double);
     unsigned long long free_mask = 0;
     for (int i = 0; i < D; ++i) if (!p->free_dof || p->free_dof[i]) free_mask |= 1ull << i;
-    const std::vector<double> Minv = sim_inverse_mass(e->T, *p, free_mask);
+    // links: a non-empty hc_sim_links runs k_body_step_linked; NULL or empty runs k_body_step as before
+    const bool linked = p->links && (p->links->n_prismatic != 0 || p->links->n_tsda != 0);
+    LinkStepArgs la{};
+    std::vector<double> link_M, link_key;
+    if (linked) sim_links_setup(e->T, *p, free_mask, la, link_M, link_key);
+    const std::vector<double> Minv = linked ? std::vector<double>() : sim_inverse_mass(e->T, *p, free_mask);
     cudaStream_t st = e->stream;
     if (e->d_sim.n != size_t(hc_ensemble::kSimSlots) * bd) { e->d_sim.alloc(size_t(hc_ensemble::kSimSlots) * bd); e->sim_q_valid = false; }
     if (e->d_simq.n != size_t(8) * B * N) { e->d_simq.alloc(size_t(8) * B * N); e->sim_q_valid = false; }
     if (e->d_minv.n != size_t(D) * D) e->d_minv.alloc(size_t(D) * D);
     // pageable sources: the runtime stages them at the call, so the host vectors may go out of scope at once
-    CUDA_CHECK(cudaMemcpyAsync(e->d_minv.p, Minv.data(), Minv.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (!linked) CUDA_CHECK(cudaMemcpyAsync(e->d_minv.p, Minv.data(), Minv.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    const hc_sim_links* L = p->links;
+    double* d_tsda_energy = nullptr;
+    if (linked) {
+        const size_t asm_n = size_t(B) * (la.n_pr * kLinkAsmJoint + la.n_tsda * kLinkAsmTsda);
+        const size_t bt = size_t(B) * la.n_tsda;
+        if (e->d_link_M.n != size_t(D) * D) e->d_link_M.alloc(size_t(D) * D);
+        if (e->d_link_asm.n != asm_n) { e->d_link_asm.alloc(asm_n); e->link_asm_valid = false; }
+        if (e->d_link_end.n != bd) { e->d_link_end.alloc(bd); e->link_asm_valid = false; }
+        if (bt > 0 && e->d_link_coef.n < 2 * bt) e->d_link_coef.alloc(2 * bt);
+        if (host && bt > 0 && L->tsda_energy && e->d_link_energy.n < bt) e->d_link_energy.alloc(bt);
+        CUDA_CHECK(cudaMemcpyAsync(e->d_link_M.p, link_M.data(), link_M.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+        if (bt > 0 && L->tsda_damping)
+            CUDA_CHECK(cudaMemcpyAsync(e->d_link_coef.p, L->tsda_damping, bt * sizeof(double), cudaMemcpyHostToDevice, st));
+        if (bt > 0 && L->tsda_stiffness)
+            CUDA_CHECK(cudaMemcpyAsync(e->d_link_coef.p + bt, L->tsda_stiffness, bt * sizeof(double), cudaMemcpyHostToDevice, st));
+        la.M = e->d_link_M.p;
+        la.asm_data = e->d_link_asm.p;
+        la.end_pose = e->d_link_end.p;
+        la.tsda_c = bt > 0 && L->tsda_damping ? e->d_link_coef.p : nullptr;
+        la.tsda_k = bt > 0 && L->tsda_stiffness ? e->d_link_coef.p + bt : nullptr;
+        d_tsda_energy = bt > 0 && L->tsda_energy ? (host ? e->d_link_energy.p : L->tsda_energy) : nullptr;
+        if (d_tsda_energy) CUDA_CHECK(cudaMemsetAsync(d_tsda_energy, 0, bt * sizeof(double), st));
+        la.tsda_energy = d_tsda_energy;
+        la.keep_asm = e->link_asm_valid && link_key == e->link_key ? 1 : 0;
+    }
     const bool has_c = p->pto_damping != nullptr, has_k = p->pto_stiffness != nullptr;
     if ((has_c || has_k) && e->d_pto.n != 2 * bd) e->d_pto.alloc(2 * bd);
     if (has_c) CUDA_CHECK(cudaMemcpyAsync(e->d_pto.p, p->pto_damping, bytes, cudaMemcpyHostToDevice, st));
@@ -2086,13 +2203,22 @@ static hc_status sim_run(hc_ensemble* e, const hc_sim_params* p, bool host, doub
     auto launch = [&](int mode, int cur) {
         a.pose_in = evp(cur); a.vel_in = evv(cur);
         a.pose_out = evp(mode == kBodyInit ? cur : cur ^ 1); a.vel_out = evv(mode == kBodyInit ? cur : cur ^ 1);
-        CUDA_CHECK(launch_body_step(a, mode, st));
+        if (linked) {
+            la.s = a;
+            CUDA_CHECK(launch_body_step_linked(la, mode, st));
+        } else {
+            CUDA_CHECK(launch_body_step(a, mode, st));
+        }
         e->prof.kernel_launches += 1;
     };
     a.keep_q = e->sim_q_valid ? 1 : 0;
     launch(kBodyInit, 0);
     e->sim_q_valid = true;
     a.keep_q = 0;
+    la.keep_asm = 0;
+    // the assembly data now belong to this run (a run without links leaves none behind)
+    e->link_asm_valid = linked;
+    if (linked) e->link_key = link_key;
 
     std::vector<double> times(static_cast<size_t>(n_rec), 0.0);
     double t = p->t0;
@@ -2134,6 +2260,14 @@ static hc_status sim_run(hc_ensemble* e, const hc_sim_params* p, bool host, doub
     CUDA_CHECK(cudaMemcpyAsync(pose, hht ? e->sim(hc_ensemble::kSimX) : evp(cur), bytes, out, st));
     CUDA_CHECK(cudaMemcpyAsync(vel, hht ? e->sim(hc_ensemble::kSimV) : evv(cur), bytes, out, st));
     if (energy && host) CUDA_CHECK(cudaMemcpyAsync(energy, d_energy, bytes, cudaMemcpyDeviceToHost, st));
+    if (linked) {
+        // the pose this run ended in: a continuation call that starts from it keeps the assembly data
+        CUDA_CHECK(cudaMemcpyAsync(e->d_link_end.p, hht ? e->sim(hc_ensemble::kSimX) : evp(cur), bytes,
+                                   cudaMemcpyDeviceToDevice, st));
+        if (d_tsda_energy && host)
+            CUDA_CHECK(cudaMemcpyAsync(L->tsda_energy, d_tsda_energy, size_t(B) * la.n_tsda * sizeof(double),
+                                       cudaMemcpyDeviceToHost, st));
+    }
     const size_t n_done_rec = size_t(done / p->record_every);
     if (rec_t && n_done_rec > 0) {
         if (host) std::memcpy(rec_t, times.data(), n_done_rec * sizeof(double));

@@ -2356,4 +2356,375 @@ cudaError_t launch_body_step(const BodyStepArgs& a, int mode, cudaStream_t st) {
     return cudaGetLastError();
 }
 
+// ---- k_body_step_linked: the chrono_compat stepper with prismatic joints and spring-dampers ----
+// ChSystem::Assemble / SolveAccelerations / ProjectOntoJoints (host/src/chrono_compat.cpp), rounded like k_body_step.
+namespace {
+struct V3 { double x, y, z; };
+__device__ __forceinline__ V3 ld3(const double* p) { return {p[0], p[1], p[2]}; }
+__device__ __forceinline__ void st3(double* p, const V3& v) { p[0] = v.x; p[1] = v.y; p[2] = v.z; }
+__device__ __forceinline__ V3 vadd(const V3& a, const V3& b) { return {add(a.x, b.x), add(a.y, b.y), add(a.z, b.z)}; }
+__device__ __forceinline__ V3 vsub(const V3& a, const V3& b) { return {sub(a.x, b.x), sub(a.y, b.y), sub(a.z, b.z)}; }
+__device__ __forceinline__ V3 vscale(const V3& a, double s) { return {mul(a.x, s), mul(a.y, s), mul(a.z, s)}; }
+__device__ __forceinline__ V3 vcross(const V3& a, const V3& b) {      // operator%
+    return {sub(mul(a.y, b.z), mul(a.z, b.y)), sub(mul(a.z, b.x), mul(a.x, b.z)), sub(mul(a.x, b.y), mul(a.y, b.x))};
+}
+__device__ __forceinline__ double vdot(const V3& a, const V3& b) { return add(add(mul(a.x, b.x), mul(a.y, b.y)), mul(a.z, b.z)); }
+__device__ __forceinline__ V3 qrot(const Quat& q, const V3& v) {       // ChQuaterniond::Rotate
+    const V3 u{q.e1, q.e2, q.e3};
+    const V3 t = vscale(vcross(u, v), 2.0);
+    return vadd(vadd(v, vscale(t, q.e0)), vcross(u, t));
+}
+__device__ __forceinline__ Quat qconj(const Quat& q) { return {q.e0, -q.e1, -q.e2, -q.e3}; }
+__device__ __forceinline__ V3 qrot_back(const Quat& q, const V3& v) { return qrot(qconj(q), v); }
+__device__ __forceinline__ Quat qnormalize(Quat p) {
+    const double n = sqrt(add(add(add(mul(p.e0, p.e0), mul(p.e1, p.e1)), mul(p.e2, p.e2)), mul(p.e3, p.e3)));
+    if (n > 0) { p.e0 = p.e0 / n; p.e1 = p.e1 / n; p.e2 = p.e2 / n; p.e3 = p.e3 / n; }
+    return p;
+}
+// state of body n of one instance (pose / vel [D], q [N][4]); n < 0 is the ground: origin, identity, at rest
+struct BodyState { V3 x, v, w; Quat q; };
+__device__ __forceinline__ BodyState body_state(int n, const double* pose, const double* vel, const double* q) {
+    if (n < 0) return {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}, {1, 0, 0, 0}};
+    return {ld3(pose + 6 * n), ld3(vel + 6 * n), ld3(vel + 6 * n + 3), load_q(q + 4 * n)};
+}
+// ProjectOntoJoints for one child: orientation q_parent rel_rot, transverse offset from the parent, slide kept
+__device__ __forceinline__ void project_child(const double* asmj, int child, int parent, double* pose, double* vel,
+                                              double* q) {
+    const BodyState B = body_state(parent, pose, vel, q);
+    const V3 off = ld3(asmj), ax = ld3(asmj + 7);
+    const V3 nax = qrot(B.q, ax);
+    const V3 rho_b = qrot_back(B.q, vsub(ld3(pose + 6 * child), B.x));
+    const double s = vdot(vsub(rho_b, off), ax);
+    const V3 rho = qrot(B.q, vadd(off, vscale(ax, s)));
+    const Quat qA = qnormalize(qmul(B.q, load_q(asmj + 3)));
+    const V3 wxr = vcross(B.w, rho);
+    const double sd = vdot(nax, vsub(vsub(ld3(vel + 6 * child), B.v), wxr));
+    store_q(q + 4 * child, qA);
+    st3(pose + 6 * child, vadd(B.x, rho));
+    cardan_xyz(qA, pose + 6 * child + 3);
+    st3(vel + 6 * child + 3, B.w);
+    st3(vel + 6 * child, vadd(vadd(B.v, wxr), vscale(nax, sd)));
+}
+}  // namespace
+
+int link_step_threads(int D, int nq) {
+    const size_t per = size_t(4 * D + nq * nq + nq) * sizeof(double);
+    int t = 64;
+    while (t > 1 && size_t(D) * D * sizeof(double) + t * per > size_t(96) * 1024) t /= 2;
+    return t;
+}
+size_t link_step_smem(int D, int nq, int threads) {
+    return (size_t(D) * D + size_t(threads) * (4 * D + nq * nq + nq)) * sizeof(double);
+}
+
+// One thread per instance, blockDim.x instances per CTA.  Shared memory: M [D][D] (staged once per CTA), then per
+// instance, element-major with stride blockDim.x: F / r [D], bias [D], per body the joint axis and rho [D], M T_c and
+// later the accelerations [D], T^T M T [nq][nq], T^T r / qdd [nq].  T is never stored: its entries are 0, 1, an axis
+// component or a component of -[rho]x, evaluated from the column's descriptor.  At most 64 threads per CTA
+// (link_step_threads); the explicit register cap keeps ptxas from spilling (it chose 96 registers and spilled under
+// __launch_bounds__(64)).
+__global__ void __maxnreg__(128) k_body_step_linked(const __grid_constant__ LinkStepArgs a, const int mode) {
+    extern __shared__ double s_mem[];
+    const BodyStepArgs& s = a.s;
+    const int D = s.D, N = s.N, nq = a.nq, nt = blockDim.x;
+    for (int i = threadIdx.x; i < D * D; i += nt) s_mem[i] = a.M[i];
+    __syncthreads();
+    const int b = blockIdx.x * nt + threadIdx.x;
+    if (b >= s.B) return;
+    const size_t o = (size_t)b * D, oq = (size_t)b * N * 4;
+    const double* sM = s_mem;
+    double* F = s_mem + (size_t)D * D + threadIdx.x;
+    double* bias = F + (size_t)D * nt;
+    double* geo = bias + (size_t)D * nt;
+    double* mt = geo + (size_t)D * nt;
+    double* A = mt + (size_t)D * nt;
+    double* rq = A + (size_t)nq * nq * nt;
+#define SH(p, i) (p)[(size_t)(i) * nt]
+    const int asm_stride = a.n_pr * kLinkAsmJoint + a.n_tsda * kLinkAsmTsda;
+    double* asm_i = a.asm_data + (size_t)b * asm_stride;
+    auto is_free = [&](int i) { return (s.free_mask >> i) & 1ull; };
+    constexpr double alpha = -0.2, gamma = 0.5 - alpha, beta = 0.25 * (1.0 - alpha) * (1.0 - alpha);
+
+    if (mode == kBodyInit) {
+        for (int n = 0; n < N; ++n) {       // k_body_step's kBodyInit
+            const double* x = s.pose_in + o + 6 * n;
+            Quat q;
+            double ang[3];
+            bool keep = false;
+            if (s.keep_q) {
+                q = load_q(s.q + oq + 4 * n);
+                cardan_xyz(q, ang);
+                keep = ang[0] == x[3] && ang[1] == x[4] && ang[2] == x[5];
+            }
+            if (!keep) {
+                q = qmul(qmul(quat_angle_axis(x[3], 1, 0, 0), quat_angle_axis(x[4], 0, 1, 0)), quat_angle_axis(x[5], 0, 0, 1));
+                store_q(s.q + oq + 4 * n, q);
+                cardan_xyz(q, ang);
+            }
+            for (int k = 0; k < 6; ++k) {
+                const double p = k < 3 ? x[k] : ang[k - 3], v = s.vel_in[o + 6 * n + k];
+                s.pose_out[o + 6 * n + k] = p; s.vel_out[o + 6 * n + k] = v;
+                if (s.sx) { s.sx[o + 6 * n + k] = p; s.sv[o + 6 * n + k] = v; }
+                if (s.x0) s.x0[o + 6 * n + k] = p;
+            }
+        }
+        bool keep = a.keep_asm != 0;
+        for (int i = 0; keep && i < D; ++i) keep = s.pose_in[o + i] == a.end_pose[o + i];
+        if (keep) return;
+        // assembly (ChLinkLockPrismatic::Initialize, ChLinkTSDA::Initialize) at the initial pose
+        const double* x = s.pose_in + o;
+        const double* qi = s.q + oq;
+        for (int j = 0; j < a.n_pr; ++j) {
+            const BodyState P = body_state(a.pr_parent[j], x, s.vel_in + o, qi);
+            const int c = a.pr_child[j];
+            double* d = asm_i + j * kLinkAsmJoint;
+            st3(d, qrot_back(P.q, vsub(ld3(x + 6 * c), P.x)));
+            store_q(d + 3, qmul(qconj(P.q), load_q(qi + 4 * c)));
+            st3(d + 7, qrot_back(P.q, V3{a.pr_axis[j][0], a.pr_axis[j][1], a.pr_axis[j][2]}));
+        }
+        for (int t = 0; t < a.n_tsda; ++t) {
+            const BodyState B1 = body_state(a.ts_b1[t], x, s.vel_in + o, qi), B2 = body_state(a.ts_b2[t], x, s.vel_in + o, qi);
+            const V3 p1{a.ts_p1[t][0], a.ts_p1[t][1], a.ts_p1[t][2]}, p2{a.ts_p2[t][0], a.ts_p2[t][1], a.ts_p2[t][2]};
+            double* d = asm_i + a.n_pr * kLinkAsmJoint + t * kLinkAsmTsda;
+            st3(d, qrot_back(B1.q, vsub(p1, B1.x)));
+            st3(d + 3, qrot_back(B2.q, vsub(p2, B2.x)));
+            const V3 l = vsub(p1, p2);
+            d[6] = a.ts_rest[t] >= 0.0 ? a.ts_rest[t] : sqrt(vdot(l, l));
+        }
+        return;
+    }
+
+    // evaluation state: Euler = the state; HHT start = the initial state; HHT step = the predictor (orientation qe)
+    const double* xin = s.pose_in + o;
+    const double* vin = s.vel_in + o;
+    const double* qev = (mode == kBodyHHTStep ? s.qe : s.q) + oq;
+
+    // generalised force: hydro + gravity - PTO damper - PTO spring, then the spring-dampers (Assemble)
+    for (int j = 0; j < D; ++j) {
+        double f = s.force[o + j];
+        const int k = j % 6;
+        if (k < 3) f = add(f, mul(s.mass[j / 6], s.g[k]));
+        const double v = vin[j];
+        if (s.pto_c) {
+            const double c = s.pto_c[o + j];
+            f = sub(f, mul(c, v));
+            if (s.energy && mode != kBodyHHTStart) s.energy[o + j] = add(s.energy[o + j], mul(mul(mul(c, v), v), s.dt));
+        }
+        if (s.pto_k) f = sub(f, mul(s.pto_k[o + j], sub(xin[j], s.x0[o + j])));
+        SH(F, j) = f;
+    }
+    for (int t = 0; t < a.n_tsda; ++t) {
+        const double* d = asm_i + a.n_pr * kLinkAsmJoint + t * kLinkAsmTsda;
+        const int i1 = a.ts_b1[t], i2 = a.ts_b2[t];
+        const BodyState B1 = body_state(i1, xin, vin, qev), B2 = body_state(i2, xin, vin, qev);
+        const V3 s1 = qrot(B1.q, ld3(d)), s2 = qrot(B2.q, ld3(d + 3));
+        const V3 dl = vsub(vadd(B1.x, s1), vadd(B2.x, s2));
+        const double len = sqrt(vdot(dl, dl));
+        if (len == 0.0) continue;
+        const V3 u = vscale(dl, 1.0 / len);
+        const double ldot = vdot(vsub(vadd(B1.v, vcross(B1.w, s1)), vadd(B2.v, vcross(B2.w, s2))), u);
+        const double c = a.tsda_c ? a.tsda_c[(size_t)b * a.n_tsda + t] : 0.0;
+        const double kk = a.tsda_k ? a.tsda_k[(size_t)b * a.n_tsda + t] : 0.0;
+        const double f = -add(mul(kk, sub(len, d[6])), mul(c, ldot));
+        if (a.tsda_energy && mode != kBodyHHTStart) {
+            double* e = a.tsda_energy + (size_t)b * a.n_tsda + t;
+            *e = add(*e, mul(mul(mul(c, ldot), ldot), s.dt));
+        }
+        if (i1 >= 0) {
+            const V3 fv = vscale(u, f), tq = vcross(s1, fv);
+            SH(F, 6 * i1) = add(SH(F, 6 * i1), fv.x); SH(F, 6 * i1 + 1) = add(SH(F, 6 * i1 + 1), fv.y);
+            SH(F, 6 * i1 + 2) = add(SH(F, 6 * i1 + 2), fv.z); SH(F, 6 * i1 + 3) = add(SH(F, 6 * i1 + 3), tq.x);
+            SH(F, 6 * i1 + 4) = add(SH(F, 6 * i1 + 4), tq.y); SH(F, 6 * i1 + 5) = add(SH(F, 6 * i1 + 5), tq.z);
+        }
+        if (i2 >= 0) {
+            const V3 fv = vscale(u, -f), tq = vcross(s2, fv);
+            SH(F, 6 * i2) = add(SH(F, 6 * i2), fv.x); SH(F, 6 * i2 + 1) = add(SH(F, 6 * i2 + 1), fv.y);
+            SH(F, 6 * i2 + 2) = add(SH(F, 6 * i2 + 2), fv.z); SH(F, 6 * i2 + 3) = add(SH(F, 6 * i2 + 3), tq.x);
+            SH(F, 6 * i2 + 4) = add(SH(F, 6 * i2 + 4), tq.y); SH(F, 6 * i2 + 5) = add(SH(F, 6 * i2 + 5), tq.z);
+        }
+    }
+    for (int j = 0; j < D; ++j) {                  // HHT: balance (1 + alpha) F_{n+1} - alpha F_n
+        if (mode == kBodyHHTStep) {
+            const double fn = s.Fn[o + j], f = SH(F, j);
+            s.Fn[o + j] = f;
+            SH(F, j) = sub(mul(1.0 + alpha, f), mul(alpha, fn));
+        } else if (mode == kBodyHHTStart) {
+            s.Fn[o + j] = SH(F, j);
+        }
+        SH(bias, j) = 0.0;
+    }
+
+    // T's data and the bias (SolveAccelerations) at the evaluation state
+    for (int j = 0; j < a.n_pr; ++j) {
+        const int c = a.pr_child[j], p = a.pr_parent[j];
+        const BodyState P = body_state(p, xin, vin, qev);
+        const V3 nax = qrot(P.q, ld3(asm_i + j * kLinkAsmJoint + 7));
+        SH(geo, 6 * c) = nax.x; SH(geo, 6 * c + 1) = nax.y; SH(geo, 6 * c + 2) = nax.z;
+        if (p < 0) continue;
+        const V3 rho = vsub(ld3(xin + 6 * c), P.x);
+        const double sd = vdot(nax, vsub(vsub(ld3(vin + 6 * c), P.v), vcross(P.w, rho)));
+        const V3 bl = vadd(vcross(P.w, vcross(P.w, rho)), vscale(vcross(P.w, nax), mul(2.0, sd)));
+        SH(geo, 6 * c + 3) = rho.x; SH(geo, 6 * c + 4) = rho.y; SH(geo, 6 * c + 5) = rho.z;
+        SH(bias, 6 * c) = bl.x; SH(bias, 6 * c + 1) = bl.y; SH(bias, 6 * c + 2) = bl.z;
+    }
+    auto T = [&](int i, int c) -> double {
+        const int bi = i / 6, k = i - 6 * bi, cb = a.col_body[c], cd = a.col_dof[c];
+        if (cd == 6) return (bi == cb && k < 3) ? SH(geo, 6 * cb + k) : 0.0;      // slide: the axis
+        if (bi == cb) return k == cd ? 1.0 : 0.0;                              // the root body's own DoF
+        if (a.parent_of[bi] != cb) return 0.0;
+        if (k == cd) return 1.0;                                               // child of this root: vA = vB, wA = wB
+        if (cd < 3 || k >= 3) return 0.0;
+        const int m = cd - 3;                                                  // -[rho]x, row k, column m
+        if (k == m) return 0.0;
+        const double r = SH(geo, 6 * bi + 3 + (3 - k - m));
+        return ((k == 0 && m == 1) || (k == 1 && m == 2) || (k == 2 && m == 0)) ? r : -r;
+    };
+    // r = rhs - M bias
+    for (int i = 0; i < D; ++i) {
+        double sacc = SH(F, i);
+        for (int j = 0; j < D; ++j) {
+            const double bj = SH(bias, j);
+            if (bj != 0.0) sacc = sub(sacc, mul(sM[i * D + j], bj));
+        }
+        SH(F, i) = sacc;
+    }
+    // T^T M T column by column (M T_c in mt), T^T r
+    for (int c = 0; c < nq; ++c) {
+        for (int i = 0; i < D; ++i) SH(mt, i) = 0.0;
+        for (int j = 0; j < D; ++j) {
+            const double t = T(j, c);
+            if (t == 0.0) continue;
+            for (int i = 0; i < D; ++i) SH(mt, i) = add(SH(mt, i), mul(sM[i * D + j], t));
+        }
+        for (int r = 0; r < nq; ++r) {
+            double sacc = 0.0;
+            for (int i = 0; i < D; ++i) {
+                const double t = T(i, r);
+                if (t != 0.0) sacc = add(sacc, mul(t, SH(mt, i)));
+            }
+            SH(A, r * nq + c) = sacc;
+        }
+    }
+    for (int r = 0; r < nq; ++r) {
+        double sacc = 0.0;
+        for (int i = 0; i < D; ++i) {
+            const double t = T(i, r);
+            if (t != 0.0) sacc = add(sacc, mul(t, SH(F, i)));
+        }
+        SH(rq, r) = sacc;
+    }
+    // solve_dense: partial pivoting, no zero pivot (the host checked that M's symmetric part is positive definite)
+    for (int k = 0; k < nq; ++k) {
+        int piv = k;
+        for (int r = k + 1; r < nq; ++r)
+            if (fabs(SH(A, r * nq + k)) > fabs(SH(A, piv * nq + k))) piv = r;
+        if (piv != k) {
+            for (int c = 0; c < nq; ++c) { const double t = SH(A, k * nq + c); SH(A, k * nq + c) = SH(A, piv * nq + c); SH(A, piv * nq + c) = t; }
+            const double t = SH(rq, k); SH(rq, k) = SH(rq, piv); SH(rq, piv) = t;
+        }
+        for (int r = k + 1; r < nq; ++r) {
+            const double m = __ddiv_rn(SH(A, r * nq + k), SH(A, k * nq + k));
+            if (m == 0.0) continue;
+            for (int c = k; c < nq; ++c) SH(A, r * nq + c) = sub(SH(A, r * nq + c), mul(m, SH(A, k * nq + c)));
+            SH(rq, r) = sub(SH(rq, r), mul(m, SH(rq, k)));
+        }
+    }
+    for (int k = nq - 1; k >= 0; --k) {
+        double sacc = SH(rq, k);
+        for (int c = k + 1; c < nq; ++c) sacc = sub(sacc, mul(SH(A, k * nq + c), SH(rq, c)));
+        SH(rq, k) = __ddiv_rn(sacc, SH(A, k * nq + k));
+    }
+    // a = bias + T qdd (into mt)
+    for (int i = 0; i < D; ++i) {
+        double sacc = SH(bias, i);
+        for (int c = 0; c < nq; ++c) {
+            const double t = T(i, c);
+            if (t != 0.0) sacc = add(sacc, mul(t, SH(rq, c)));
+        }
+        SH(mt, i) = sacc;
+    }
+    const double h = s.dt;
+    auto rec = [&](const double* p, const double* v) {
+        for (int i = 0; i < D; ++i) {
+            if (s.rec_pose) s.rec_pose[o + i] = p[i];
+            if (s.rec_vel) s.rec_vel[o + i] = v[i];
+        }
+    };
+    if (mode == kBodyEuler) {
+        double* po = s.pose_out + o;
+        double* vo = s.vel_out + o;
+        double* qs = s.q + oq;
+        for (int n = 0; n < N; ++n) {
+            double v[6];
+            for (int k = 0; k < 6; ++k) v[k] = is_free(6 * n + k) ? add(vin[6 * n + k], mul(h, SH(mt, 6 * n + k))) : 0.0;
+            const Quat q = rotate_by(load_q(qs + 4 * n), mul(v[3], h), mul(v[4], h), mul(v[5], h));
+            store_q(qs + 4 * n, q);
+            for (int k = 0; k < 3; ++k) po[6 * n + k] = add(xin[6 * n + k], mul(v[k], h));
+            cardan_xyz(q, po + 6 * n + 3);
+            for (int k = 0; k < 6; ++k) vo[6 * n + k] = v[k];
+        }
+        for (int j = 0; j < a.n_pr; ++j) project_child(asm_i + j * kLinkAsmJoint, a.pr_child[j], a.pr_parent[j], po, vo, qs);
+        rec(po, vo);
+        return;
+    }
+    double* sx = s.sx + o;
+    double* sv = s.sv + o;
+    double* qs = s.q + oq;
+    if (mode == kBodyHHTStep) {                    // corrector from the saved state x_n, v_n, q_n
+        for (int n = 0; n < N; ++n) {
+            double dth[3];
+            for (int k = 0; k < 6; ++k) {
+                const double a0 = s.an[o + 6 * n + k], a1 = SH(mt, 6 * n + k);
+                const double v = sv[6 * n + k];
+                const double dv = mul(h, add(mul(1.0 - gamma, a0), mul(gamma, a1)));
+                const double dx = add(mul(h, v), mul(mul(h, h), add(mul(0.5 - beta, a0), mul(beta, a1))));
+                const bool fr = is_free(6 * n + k);
+                if (k < 3) {
+                    if (fr) { sx[6 * n + k] = add(sx[6 * n + k], dx); sv[6 * n + k] = add(v, dv); } else sv[6 * n + k] = 0.0;
+                } else {
+                    if (fr) { dth[k - 3] = dx; sv[6 * n + k] = add(v, dv); } else { dth[k - 3] = 0.0; sv[6 * n + k] = 0.0; }
+                }
+            }
+            const Quat q = rotate_by(load_q(qs + 4 * n), dth[0], dth[1], dth[2]);
+            store_q(qs + 4 * n, q);
+            cardan_xyz(q, sx + 6 * n + 3);
+        }
+        for (int j = 0; j < a.n_pr; ++j) project_child(asm_i + j * kLinkAsmJoint, a.pr_child[j], a.pr_parent[j], sx, sv, qs);
+        rec(sx, sv);
+    }
+    // predictor of the next step: x* = x + h v + h^2/2 a,  v* = v + h a,  q* = rotate_by(q, h w + h^2/2 alpha)
+    double* po = s.pose_out + o;
+    double* vo = s.vel_out + o;
+    double* qp = s.qe + oq;
+    const double hh2 = mul(mul(0.5, h), h);
+    for (int i = 0; i < D; ++i) s.an[o + i] = SH(mt, i);
+    for (int n = 0; n < N; ++n) {
+        double an[6], v[6];
+        for (int k = 0; k < 6; ++k) { an[k] = SH(mt, 6 * n + k); v[k] = sv[6 * n + k]; }
+        for (int k = 0; k < 3; ++k) po[6 * n + k] = add(add(sx[6 * n + k], mul(v[k], h)), mul(an[k], hh2));
+        const Quat qe = rotate_by(load_q(qs + 4 * n), add(mul(v[3], h), mul(an[3], hh2)), add(mul(v[4], h), mul(an[4], hh2)),
+                                  add(mul(v[5], h), mul(an[5], hh2)));
+        store_q(qp + 4 * n, qe);
+        cardan_xyz(qe, po + 6 * n + 3);
+        for (int k = 0; k < 6; ++k) vo[6 * n + k] = add(v[k], mul(an[k], h));
+    }
+    for (int j = 0; j < a.n_pr; ++j) project_child(asm_i + j * kLinkAsmJoint, a.pr_child[j], a.pr_parent[j], po, vo, qp);
+#undef SH
+}
+
+cudaError_t launch_body_step_linked(const LinkStepArgs& a, int mode, cudaStream_t st) {
+    const int threads = link_step_threads(a.s.D, a.nq);
+    const size_t smem = link_step_smem(a.s.D, a.nq, threads);
+    static bool attr_set[64] = {};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (smem > 48 * 1024 && !attr_set[dev & 63]) {      // link_step_threads keeps smem <= 96 KB + M (<= 18 KB)
+        cudaError_t e = cudaFuncSetAttribute(k_body_step_linked, cudaFuncAttributeMaxDynamicSharedMemorySize, 120 * 1024);
+        if (e != cudaSuccess) return e;
+        attr_set[dev & 63] = true;
+    }
+    k_body_step_linked<<<(a.s.B + threads - 1) / threads, threads, smem, st>>>(a, mode);
+    return cudaGetLastError();
+}
+
 }  // namespace hc

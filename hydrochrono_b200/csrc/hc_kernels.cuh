@@ -293,4 +293,35 @@ struct BodyStepArgs {
 };
 cudaError_t launch_body_step(const BodyStepArgs& a, int mode, cudaStream_t st);
 
+// ---- device-side stepping with prismatic joints and translational spring-dampers (k_body_step_linked) ----
+// The same modes, slots and ping-pong pairs as k_body_step (the BodyStepArgs fields keep their meaning; Minv is unused).
+// Per instance and step: generalised force (hydro, gravity, per-DoF PTO, spring-dampers), T and the bias from the
+// evaluation state, (T^T M T) qdd = T^T (rhs - M bias) by partial-pivot elimination, a = bias + T qdd, the scheme's
+// update and the projection of every child onto its joint.
+constexpr int kMaxLinkTsda = 16;          // HC_SIM_MAX_TSDA
+constexpr int kLinkAsmJoint = 10;         // per joint: offset in the parent frame [3], relative rotation [4], axis in the parent frame [3]
+constexpr int kLinkAsmTsda = 7;           // per spring-damper: body-frame points [3] + [3], rest length
+struct LinkStepArgs {
+    BodyStepArgs s;
+    const double* M;          // [D][D] diag(m, I) + A_inf over every DoF
+    double* asm_data;         // [B][n_pr kLinkAsmJoint + n_tsda kLinkAsmTsda] assembly data (kBodyInit derives it)
+    const double* end_pose;   // [B][D] kBodyInit with keep_asm: the pose the previous linked call ended in
+    const double* tsda_c;     // [B][n_tsda] or null
+    const double* tsda_k;     // [B][n_tsda] or null
+    double* tsda_energy;      // [B][n_tsda] or null: += c ldot ldot dt with the evaluation state's ldot
+    int n_pr, n_tsda, nq;
+    int keep_asm;             // kBodyInit: keep the assembly data of an instance whose pose equals end_pose bit for bit
+    int parent_of[kMaxBodies];        // -2: root body, -1: child of ground, else the parent's index
+    int joint_of[kMaxBodies];         // index of the joint whose child the body is, or -1
+    int pr_child[kMaxBodies], pr_parent[kMaxBodies];
+    double pr_axis[kMaxBodies][3];    // unit axis, world frame at assembly
+    int ts_b1[kMaxLinkTsda], ts_b2[kMaxLinkTsda];
+    double ts_p1[kMaxLinkTsda][3], ts_p2[kMaxLinkTsda][3], ts_rest[kMaxLinkTsda];
+    signed char col_body[6 * kMaxBodies], col_dof[6 * kMaxBodies];   // column c of T: a root DoF (body, 0..5) or a slide (child, 6)
+};
+// Dynamic shared memory of one CTA of `threads` instances: M plus the per-instance scratch.
+size_t link_step_smem(int D, int nq, int threads);
+int link_step_threads(int D, int nq);
+cudaError_t launch_body_step_linked(const LinkStepArgs& a, int mode, cudaStream_t st);
+
 }  // namespace hc

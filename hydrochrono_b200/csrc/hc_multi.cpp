@@ -241,6 +241,15 @@ hc_status hc_multi_ensemble_simulate(hc_multi_ensemble* m, const hc_sim_params* 
         hc_sim_params q = *p;
         if (p->pto_damping) q.pto_damping = p->pto_damping + off;
         if (p->pto_stiffness) q.pto_stiffness = p->pto_stiffness + off;
+        hc_sim_links l{};
+        if (p->links) {            // per-instance spring-damper coefficients and energies: the shard's rows
+            l = *p->links;
+            const size_t toff = size_t(k.first) * size_t(l.n_tsda > 0 ? l.n_tsda : 0);
+            if (l.tsda_damping) l.tsda_damping += toff;
+            if (l.tsda_stiffness) l.tsda_stiffness += toff;
+            if (l.tsda_energy) l.tsda_energy += toff;
+            q.links = &l;
+        }
         int done = 0;
         // only the first shard writes the (shared) record times
         const hc_status s = hc_ensemble_simulate_strided(k.ens, &q, pose + off, vel + off, k.first == 0 ? rec_t : nullptr,

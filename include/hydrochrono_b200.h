@@ -288,8 +288,9 @@ HC_API hc_status hc_waves_kinematics_at_time_device(hc_ensemble* e, double t, in
  * kernel (k_body_step), no host synchronisation inside the loop.  Rigid bodies with 6 DoF each, every DoF free or locked
  * to ground; forces = hydro + m g on translations + an optional linear PTO per instance and DoF,
  * -k (x - x_init) - c v.  Mass matrix = diag(m, m, m, Ixx, Iyy, Izz) per body + the infinite-frequency added mass
- * (hc_added_mass), restricted to the free DoFs, inverted once on the host per call.  Constrained multibody systems
- * (joints between moving bodies, spring-damper geometry, contact) are not covered: step those with Chrono.
+ * (hc_added_mass), restricted to the free DoFs, inverted once on the host per call.  Prismatic joints and translational
+ * spring-dampers (the RM3 float / spar pair and its PTO) are covered through hc_sim_params.links (below).  Revolute
+ * joints, rotational spring-dampers, chains of joints, contact and mooring are not covered: step those with Chrono.
  * The schemes follow the chrono_compat stepper (hydrochrono_b200/host/src/chrono_compat.cpp) operation for operation:
  *   scheme 0, linearised Euler (ChSystem::StepEnd): forces at (t_n, x_n, v_n); v += dt a (locked DoFs: v = 0);
  *     x += dt v; q <- normalize(QuatFromAngleAxis(|w dt|, w / |w|) q).
@@ -310,7 +311,56 @@ HC_API hc_status hc_waves_kinematics_at_time_device(hc_ensemble* e, double t, in
  * Errors of the force path (HC_ERR_ETA_WINDOW, HC_ERR_DUPLICATE_TIME, ...; all detected when a step is enqueued) end the
  * run with that status: *steps_done = completed steps, pose / vel hold the state after the last completed step, the
  * records and energy cover the completed steps.  HC_ERR_INVALID: n_steps < 1, record_every < 1, dt <= 0, mass or
- * inertia NULL, pose or vel NULL, a singular free-DoF mass matrix. */
+ * inertia NULL, pose or vel NULL, a singular free-DoF mass matrix.
+ *
+ * Joints and spring-dampers (links != NULL with at least one joint or spring-damper; a NULL or empty links struct runs
+ * the path above unchanged, bit for bit).  They follow the chrono_compat stepper's reduced coordinates
+ * (ChSystem::Assemble / SolveAccelerations / ProjectOntoJoints) operation for operation, in one device kernel
+ * (k_body_step_linked):
+ *   - Prismatic joint to a moving parent B: the child A keeps one slide DoF along the joint axis n.  The columns of T
+ *     are the free DoFs of every root body (a body that is nobody's child), then one slide per child;
+ *     vA = vB + wB x rho + sd n, wA = wB (rho = xA - xB), with the bias wB x (wB x rho) + 2 sd wB x n.  Per step
+ *     (T^T M T) qdd = T^T (rhs - M bias) is solved by partial-pivot Gaussian elimination and a = bias + T qdd, with
+ *     M = diag(m, m, m, Ixx, Iyy, Izz) per body + A_inf over all 6N DoFs.
+ *   - Prismatic joint to ground (parent = -1): vA = sd n, wA = 0 (the reference's sphere demos).
+ *   - After every position / velocity update (the Euler update, the HHT predictor and the HHT corrector) each child is
+ *     projected onto its joint: orientation q_parent rel_rot, transverse offset from the parent, slide kept, velocity
+ *     vB + wB x rho + sd n.  The initial state is not projected.
+ *   - Spring-damper: force -(k (l - rest) + c dl/dt) along the line between the two attachment points at the
+ *     evaluation state, applied with its moment s x f to both bodies.  tsda_energy = sum over the call's steps of
+ *     c (dl/dt)^2 dt with dl/dt of that step's force evaluation (the convention of pto_energy).
+ *   - Assembly data (each joint's offset in the parent frame, relative rotation and axis in the parent frame; each
+ *     spring-damper's body-frame points and rest length) are derived per instance from its initial pose.  They are
+ *     kept by a continuation call -- the instance's given pose equals, bit for bit, the pose the previous call ended
+ *     in, and the links are the same -- so that Euler with links split into calls is bitwise identical to one call;
+ *     otherwise, and after hc_ensemble_reset, they are derived again.
+ *   - free_dof selects the DoFs of root bodies; pto_damping / pto_stiffness and gravity add to the generalised force
+ *     before it is projected through T^T.
+ * HC_ERR_INVALID (checked on the host at the call, before anything runs): a body index out of range; child == parent;
+ * a second joint on one child; a chain (a parent that is itself a child); a zero axis; more than HC_SIM_MAX_TSDA
+ * spring-dampers; a spring-damper with body1 == body2 or between ground and ground; a jointed child with a locked DoF;
+ * a mass matrix diag(m, I) + A_inf whose symmetric part is not positive definite (which keeps every T^T M T
+ * nonsingular).
+ * Callers must zero-initialise hc_sim_params (hc_sim_params p{} in C++, memset in C): fields added at its end read as
+ * "absent" when zero. */
+#define HC_SIM_MAX_TSDA 16
+typedef struct hc_sim_prismatic {   /* ChLinkLockPrismatic */
+    int child, parent;              /* body indices; parent = -1: ground */
+    double axis[3];                 /* joint axis in the world frame at assembly (the z axis of the joint frame) */
+} hc_sim_prismatic;
+typedef struct hc_sim_tsda {        /* ChLinkTSDA */
+    int body1, body2;               /* body index, -1: ground */
+    double point1[3], point2[3];    /* attachment points, world frame at assembly */
+    double rest_length;             /* < 0: the length at assembly (ChLinkTSDA::Initialize) */
+} hc_sim_tsda;
+typedef struct hc_sim_links {
+    int n_prismatic, n_tsda;
+    const hc_sim_prismatic* prismatic;
+    const hc_sim_tsda* tsda;
+    const double* tsda_damping;     /* [B][n_tsda] or NULL (0) */
+    const double* tsda_stiffness;   /* [B][n_tsda] or NULL (0) */
+    double* tsda_energy;            /* [B][n_tsda] out or NULL; host or device memory, matching the call variant */
+} hc_sim_links;
 typedef struct hc_sim_params {
     int scheme;                 /* 0 = linearised Euler, 1 = HHT-alpha (alpha = -0.2) */
     double t0, dt;
@@ -321,6 +371,7 @@ typedef struct hc_sim_params {
     const int* free_dof;        /* [6N] 1 free / 0 locked to ground; NULL = all free */
     const double* pto_damping;  /* [B][6N] or NULL */
     const double* pto_stiffness;/* [B][6N] or NULL; spring about the instance's initial pose */
+    const hc_sim_links* links;  /* NULL: free / ground-locked bodies only */
 } hc_sim_params;
 /* Host buffers: pose / vel [B][6N] (in: initial state, out: final state), rec_t [n_rec], rec_pose / rec_vel
  * [n_rec][B][6N], pto_energy [B][6N].  Records go through a device buffer of bounded size, copied out in chunks.
@@ -450,7 +501,8 @@ HC_API hc_status hc_multi_waves_kinematics_at_time(hc_multi_ensemble* m, double 
                                                    double mwl, int wheeler_stretching,
                                                    double* eta, double* velocity, double* acceleration);
 /* hc_ensemble_simulate for every shard at once: host arrays in global instance order (pose / vel / pto_energy [B][6N],
- * rec_pose / rec_vel [n_rec][B][6N], pto_* of the params [B][6N]).  Each shard runs its whole loop on its own worker
+ * rec_pose / rec_vel [n_rec][B][6N], pto_* of the params [B][6N], tsda_damping / tsda_stiffness / tsda_energy of the
+ * links [B][n_tsda]).  Each shard runs its whole loop on its own worker
  * thread, with no cross-shard barrier per step.  *steps_done = the fewest steps any shard completed. */
 HC_API hc_status hc_multi_ensemble_simulate(hc_multi_ensemble* m, const hc_sim_params* p, double* pose, double* vel,
                                             double* rec_t, double* rec_pose, double* rec_vel, double* pto_energy,
